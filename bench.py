@@ -18,6 +18,12 @@ polus_b200.training.ClassifierTrainer.train_step on one synthetic batch per GPU.
 `configs`  : device-resident throughput of BASELINE.json configs[3] (cross-encoder S=512) and configs[4] (BERT-large
            dims S=512), data parallel over the same N GPUs.
 `dp_parity`: N > 1 only -- N ranks on slices of a global batch vs one rank on the whole batch (tests/dp_parity.py).
+
+--dump-outputs DIR: each timed region starts from the model's initial weights (restore_state) and, after them, rank 0
+writes the loss of each region's last step as DIR/<name>.npy (dump_outputs), so that two builds run with the same
+arguments (identical seeded inputs and starting weights) can be compared output for output.  Two runs of one build
+still differ in the last bits of every step's float-atomic reductions, and the steps of a region compound that: on a
+B200 the losses agree to <1e-7 relative after 5 steps at batch 32, and to ~1e-6..1e-5 after 20 steps at batch 256.
 """
 import argparse
 import json
@@ -221,6 +227,34 @@ class Timer:
         return ms.value, _lib.call("polus_launch_count") - l0, float(last)
 
 
+def initial_state(trainer, x):
+    """Host copy of every trainable weight before the first training step.  A forward pass without training builds the
+    lazily created variables (NER head, CRF) first; it updates nothing."""
+    trainer.model(**x, training=False)
+    return [(w, w.numpy()) for w in trainer.model.trainable_weights]
+
+
+def restore_state(trainer, start):
+    """Back to the weights of initial_state() with zeroed Adam moments.  The gradient reductions add with float atomics,
+    so each training step differs from run to run in the last bits and successive steps compound that; timed regions
+    that start from this state start from the same weights on every run.  The step counter keeps its value: the
+    learning-rate schedule and the dropout streams go on as they would without the restore."""
+    from polus_b200 import _lib, device
+    for w, value in start:
+        w.assign(value)
+    for slot in trainer.optimizer.variables():   # Adam's first and second moments
+        _lib.call("polus_memset", slot.ptr, 0, slot.nbytes, device.stream())
+    device.device_sync()
+
+
+def dump_outputs(out_dir, losses):
+    """What a caller of the timed train steps receives: the loss of the last step of each timed region, as
+    DIR/loss_<region>.npy (float32, shape (1,))."""
+    os.makedirs(out_dir, exist_ok=True)
+    for region, value in losses.items():
+        np.save(os.path.join(out_dir, f"loss_{region}.npy"), np.asarray([value], np.float32))
+
+
 def to_device(batches):
     from polus_b200 import tensor
     out = []
@@ -289,6 +323,7 @@ def run_ours(args):
         dbg(f"dp parity: {dp_parity}")
 
     trainer, batches, _, _, _ = build_workload("ner_base", args.batch)
+    start = initial_state(trainer, batches[0][0]) if args.dump_outputs else None
     dbg("model built")
     for i in range(max(args.warmup, 3)):
         loss = trainer.train_step(*batches[i % len(batches)])
@@ -309,9 +344,13 @@ def run_ours(args):
         if i % 10 == 9:
             float(last)
     dbg("pre-heat done")
+    if start is not None:
+        restore_state(trainer, start)
     sampler = ClockSampler(local_rank) if rank == 0 else None
     ms_dev, launches, loss_dev = timed(trainer, dev_batches, args.steps)
     dbg("timed (resident) done")
+    if start is not None:
+        restore_state(trainer, start)
     ms_e2e, _, loss_e2e = timed(trainer, batches, args.steps)
     h2d = trainer.last_h2d_bytes  # bytes the public API copied host -> device for ONE step of the e2e region
     dbg("timed (e2e) done")
@@ -320,6 +359,8 @@ def run_ours(args):
     if not (np.isfinite(loss_dev) and np.isfinite(loss_e2e)):
         # a step that diverged runs on NaNs (less switching, higher clocks): its timing is not a measurement
         raise RuntimeError(f"bench: non-finite training loss (resident {loss_dev}, e2e {loss_e2e}) on rank {rank}")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"resident": loss_dev, "e2e": loss_e2e})
 
     # ---- roofline of the dominant kernel family (tcgen05 GEMMs, ~all FLOPs of the step)
     # (1) one op-by-op step counts the launches and their algorithmic FLOPs (2mnk each);
@@ -479,7 +520,7 @@ def run_ours(args):
     if not args.no_extra_configs:
         extra = {}
         for name, b in (("cfg4", args.cfg4_batch), ("cfg5", args.cfg5_batch)):
-            r = quick_config(name, b, max(5, args.steps // 2), timer, world)
+            r = quick_config(name, b, args.steps, timer, world)
             extra[name + "_seq_s"] = r["seq_s"]
             extra[name] = r
             dbg(f"{name} done: {r['seq_s']:.1f} seq/s")
@@ -536,7 +577,13 @@ def main():
     ap.add_argument("--no-extra-configs", action="store_true", help="skip the cfg4 / cfg5 (S=512) throughput lines")
     ap.add_argument("--cfg4-batch", type=int, default=64)
     ap.add_argument("--cfg5-batch", type=int, default=32)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="start each timed region from the initial weights and write "
+                    "the loss of each region's last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what --impl ours computed")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -120,22 +120,20 @@ def test_warmup_scheduler_matches_hf_torch_polynomial_schedule():
     """polus/schedulers.py:5-23 = HF `WarmUp` over Keras `PolynomialDecay(power=1, end_learning_rate=1e-7)`.  TensorFlow is
     not installable here, but transformers ships the torch twin of the same schedule
     (`get_polynomial_decay_schedule_with_warmup(lr_end=1e-7, power=1.0)`): an implementation that is neither the oracle's
-    nor the product's.  Both must follow it step by step (the device evaluates the same closed form inside polus_adam)."""
-    import torch
-    from transformers.optimization import get_polynomial_decay_schedule_with_warmup
+    nor the product's.  Both must follow it step by step (the device evaluates the same closed form inside polus_adam).
+    Its learning rates are stored in tests/golden/hf_polynomial_warmup.npz (generator: tests/golden/make_schedule_golden.py)."""
     from oracle import numpy_ref as R
     from polus_b200.schedulers import warmup_scheduler
-    for n_steps, lr in ((200, 3e-4), (1000, 5e-5), (37, 1e-3)):
+    with np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "hf_polynomial_warmup.npz")) as z:
+        cases = [(int(n), float(lr), z[f"lrs_{i}"]) for i, (n, lr) in enumerate(zip(z["n_steps"], z["lr"]))]
+    assert [(n, lr) for n, lr, _ in cases] == [(200, 3e-4), (1000, 5e-5), (37, 1e-3)]
+    for n_steps, lr, hf_lrs in cases:
         sched = warmup_scheduler(n_steps, lr)
-        opt = torch.optim.SGD([torch.nn.Parameter(torch.zeros(1))], lr=lr)
-        hf = get_polynomial_decay_schedule_with_warmup(opt, num_warmup_steps=int(n_steps * 0.1), num_training_steps=n_steps,
-                                                       lr_end=1e-7, power=1.0)
+        assert hf_lrs.shape == (n_steps + 1,)
         for step in range(n_steps + 1):
-            want = hf.get_last_lr()[0]
+            want = float(hf_lrs[step])
             assert abs(sched(step) - want) <= 1e-12 * max(1.0, want / 1e-7), (n_steps, step, sched(step), want)
             assert abs(R.warmup_schedule_lr(step, n_steps, lr) - want) <= 1e-12 * max(1.0, want / 1e-7)
-            opt.step()
-            hf.step()
 
 
 def test_warmup_scheduler_matches_oracle():
@@ -522,6 +520,16 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": "sequences/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     silent = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=root, env=dict(os.environ, RANK="1", WORLD_SIZE="2"))
     assert silent.returncode == 0 and silent.stdout.strip() == ""
+
+
+def test_bench_dump_outputs_writes_the_last_losses_as_float32(tmp_path):
+    """`bench.py --dump-outputs DIR`: one float32 .npy of shape (1,) per timed region, named after the region."""
+    import bench
+    bench.dump_outputs(str(tmp_path / "out"), {"resident": 1.5, "e2e": 2.25})
+    assert sorted(os.listdir(tmp_path / "out")) == ["loss_e2e.npy", "loss_resident.npy"]
+    for name, value in (("loss_resident.npy", 1.5), ("loss_e2e.npy", 2.25)):
+        a = np.load(tmp_path / "out" / name)
+        assert a.dtype == np.float32 and a.tolist() == [value]
 
 
 def test_bioc_sequence_decoder_flow_and_strict_evaluation():

@@ -1,13 +1,18 @@
 """Tokenisation parity (north_star: "tokenisation ... must be bit-exact"): polus_b200.tokenization against the Rust
 `tokenizers` library -- the engine behind the BertTokenizerFast the reference calls (polus/models.py:275-284) -- on
 random vocabularies, Unicode text, sentence pairs, truncation and fixed-length padding.  Sentences of the reference's own
-tests (tests/test_models.py:16, tests/test_data.py:374-376) are included."""
+tests (tests/test_models.py:16, tests/test_data.py:374-376) are included.  The library's encodings of these seeded
+inputs are stored in tests/golden/wordpiece_tokenizers.npz (generator: tests/golden/make_tokenizer_golden.py), so the
+comparison needs no tokenizer package."""
+import hashlib
+import os
 import random
 
 import numpy as np
 import pytest
 
-tokenizers = pytest.importorskip("tokenizers")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "wordpiece_tokenizers.npz")
+MAX_LENGTH = 50
 
 REFERENCE_SENTENCES = [
     "Hello, my dog is cute",
@@ -59,38 +64,52 @@ def make_text(rng, vocab_words):
     return "".join(parts)
 
 
-def library_tokenizer(vocab, lowercase, max_length):
-    from tokenizers import Tokenizer, models, normalizers, pre_tokenizers, processors
-    tok = Tokenizer(models.WordPiece(vocab, unk_token="[UNK]", max_input_chars_per_word=100))
-    tok.add_special_tokens(["[PAD]", "[UNK]", "[CLS]", "[SEP]", "[MASK]"])
-    tok.normalizer = normalizers.BertNormalizer(clean_text=True, handle_chinese_chars=True, strip_accents=None, lowercase=lowercase)
-    tok.pre_tokenizer = pre_tokenizers.BertPreTokenizer()
-    tok.post_processor = processors.BertProcessing(("[SEP]", vocab["[SEP]"]), ("[CLS]", vocab["[CLS]"]))
-    tok.enable_truncation(max_length=max_length, strategy="longest_first")
-    tok.enable_padding(length=max_length, pad_id=vocab["[PAD]"], pad_token="[PAD]", pad_type_id=0)
-    return tok
+def seeded_inputs(lowercase):
+    """The vocabulary, texts and sentence pairs the golden encodings were made from."""
+    rng = random.Random(1234 + lowercase)
+    vocab = make_vocab(rng)
+    words = [w for w in vocab if not w.startswith("##") and not w.startswith("[")]
+    texts = REFERENCE_SENTENCES + [make_text(rng, words) for _ in range(400)]
+    pairs = [(make_text(rng, words), make_text(rng, words)) for _ in range(200)]  # query / document (polus.ir cross-encoder)
+    return vocab, texts, pairs
+
+
+def inputs_digest(texts, pairs):
+    return hashlib.sha256("\x1f".join(texts + [s for p in pairs for s in p]).encode("utf-8")).hexdigest()
+
+
+def golden_key(lowercase):
+    return "lower" if lowercase else "cased"
+
+
+def padded(ids, n_first, vocab):
+    """(input_ids, token_type_ids, attention_mask) padded to MAX_LENGTH from the unpadded ids and the first segment's length."""
+    n, pad = len(ids), MAX_LENGTH - len(ids)
+    return list(ids) + [vocab["[PAD]"]] * pad, [0] * n_first + [1] * (n - n_first) + [0] * pad, [1] * n + [0] * pad
+
+
+def golden_encodings(z, key, kind, vocab):
+    ids, lens, first = (z[f"{key}_{kind}_{f}"].astype(np.int64) for f in ("ids", "len", "first"))
+    ends = np.cumsum(lens)
+    return [padded(ids[e - n:e].tolist(), int(n0), vocab) for e, n, n0 in zip(ends, lens, first)]
 
 
 @pytest.mark.parametrize("lowercase", [True, False])
 def test_wordpiece_bit_exact_against_tokenizers(lowercase):
     from polus_b200.tokenization import BertWordPieceTokenizer
-    rng = random.Random(1234 + lowercase)
-    vocab = make_vocab(rng)
-    words = [w for w in vocab if not w.startswith("##") and not w.startswith("[")]
-    max_length = 50
-    ref = library_tokenizer(vocab, lowercase, max_length)
+    vocab, texts, pairs = seeded_inputs(lowercase)
+    key = golden_key(lowercase)
+    with np.load(GOLDEN) as z:
+        assert inputs_digest(texts, pairs) == str(z[f"{key}_inputs_sha256"]), "seeded inputs differ from the golden file's"
+        singles, doubles = golden_encodings(z, key, "single", vocab), golden_encodings(z, key, "pair", vocab)
+    assert len(singles) == len(texts) and len(doubles) == len(pairs)
     ours = BertWordPieceTokenizer(vocab, lowercase=lowercase)
-    texts = REFERENCE_SENTENCES + [make_text(rng, words) for _ in range(400)]
-    for t in texts:
-        e = ref.encode(t)
-        o = ours(t, max_length=max_length, padding="max_length", truncation=True)
-        assert o["input_ids"] == e.ids, repr(t)
-        assert o["token_type_ids"] == e.type_ids and o["attention_mask"] == e.attention_mask, repr(t)
-    for _ in range(200):  # query / document pairs (polus.ir cross-encoder input)
-        a, b = make_text(rng, words), make_text(rng, words)
-        e = ref.encode(a, b)
-        o = ours(a, b, max_length=max_length, padding="max_length", truncation=True)
-        assert (o["input_ids"], o["token_type_ids"], o["attention_mask"]) == (e.ids, e.type_ids, e.attention_mask), (a, b)
+    for t, e in zip(texts, singles):
+        o = ours(t, max_length=MAX_LENGTH, padding="max_length", truncation=True)
+        assert (o["input_ids"], o["token_type_ids"], o["attention_mask"]) == e, repr(t)
+    for (a, b), e in zip(pairs, doubles):
+        o = ours(a, b, max_length=MAX_LENGTH, padding="max_length", truncation=True)
+        assert (o["input_ids"], o["token_type_ids"], o["attention_mask"]) == e, (a, b)
 
 
 def test_batch_call_shape_matches_reference_usage():
