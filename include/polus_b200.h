@@ -201,22 +201,11 @@ int polus_attention_supported(int S, int head_dim);           /* head_dim 64, 32
 size_t polus_attention_keepbits_words(int B, int S, int nh);   /* uint32 words of the dropout keep-bit buffer */
 int polus_attention_fwd(const polus_bf16_t* d_qkv, const int32_t* d_mask, int B, int S, int nh, int head_dim,
                         float p_drop, uint64_t seed, uint32_t site, const uint32_t* d_step, polus_bf16_t* d_ctx,
-                        float* d_lse, uint32_t* d_keepbits, uint32_t* d_keepbits_alt, const uint32_t* d_ready,
-                        void* stream);
+                        float* d_lse, uint32_t* d_keepbits, void* stream);
 int polus_attention_bwd(const polus_bf16_t* d_qkv, const int32_t* d_mask, const polus_bf16_t* d_ctx,
                         const polus_bf16_t* d_dctx, const float* d_lse, int B, int S, int nh, int head_dim,
                         float p_drop, uint64_t seed, uint32_t site, const uint32_t* d_step,
-                        const uint32_t* d_keepbits, const uint32_t* d_keepbits_alt, polus_bf16_t* d_dqkv,
-                        float* d_gbias_qkv, void* stream);
-/* Dropout keep bits of the attention probabilities drawn AHEAD of time (same Philox4x32-10 counters as the forward
- * kernel's own path): fills the buffer of step *d_step + step_offset -- d_keepbits for even steps, d_keepbits_alt
- * for odd ones -- and then sets d_ready[step & 1] = step + 1.  A forward launch that finds its step published reads
- * the bits instead of drawing them (56 % of its instructions); otherwise it draws them itself, so results never
- * depend on whether this ran.  Meant for a low-priority stream inside the captured step (d_keepbits_alt / d_ready
- * may be NULL in the fwd / bwd calls: one buffer, drawn in the forward). */
-int polus_attention_keepbits(uint32_t* d_keepbits, uint32_t* d_keepbits_alt, uint32_t* d_ready, int B, int S, int nh,
-                             float p_drop, uint64_t seed, uint32_t site, const uint32_t* d_step,
-                             uint32_t step_offset, void* stream);
+                        const uint32_t* d_keepbits, polus_bf16_t* d_dqkv, float* d_gbias_qkv, void* stream);
 /* d_gbias_qkv (may be NULL): [3*nh*head_dim] fp32, += column sums of d_dqkv -- the BiasAddGrad of the QKV projection
  * (polus/training.py:185), taken from the tiles while they are still in shared memory. */
 

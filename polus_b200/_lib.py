@@ -99,9 +99,8 @@ _SIGS = {
     "polus_softmax_bwd": [p, p, i32, i32, i32, i32, f32, f32, u64, u32, p, p],
     "polus_attention_supported": [i32, i32],
     "polus_attention_keepbits_words": [i32, i32, i32],
-    "polus_attention_fwd": [p, p, i32, i32, i32, i32, f32, u64, u32, p, p, p, p, p, p, p],
-    "polus_attention_bwd": [p, p, p, p, p, i32, i32, i32, i32, f32, u64, u32, p, p, p, p, p, p],
-    "polus_attention_keepbits": [p, p, p, i32, i32, i32, f32, u64, u32, p, u32, p],
+    "polus_attention_fwd": [p, p, i32, i32, i32, i32, f32, u64, u32, p, p, p, p, p],
+    "polus_attention_bwd": [p, p, p, p, p, i32, i32, i32, i32, f32, u64, u32, p, p, p, p, p],
     "polus_act_bwd_colsum": [p, p, i32, i32, i32, p, p, p, p],
     "polus_colsum_ws_floats": [i32],
     "polus_dropout": [p, p, i64, f32, u64, u32, p, p],

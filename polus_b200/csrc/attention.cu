@@ -47,17 +47,9 @@ struct AttnParams {
     const int32_t* mask;   // [B,S] or null
     float* lse;            // [B,nh,S]
     uint32_t* keepbits;    // [B*nh*S][S/32] dropout keep bits (forward writes, backward reads); null when p = 0
-    uint32_t* keepbits_alt;  // second buffer: steps with odd *d_step use it (null: one buffer for every step)
-    const uint32_t* ready;   // [2] ready[s & 1] == s + 1: the buffer of step s was filled ahead of time by
-                             // attn_keepbits_kernel (polus_attention_keepbits); null / mismatch: the forward draws them itself
     float* gbias;          // backward: [3H] bias gradient of the QKV projection += column sums of dqkv; may be null
     int pf_stride;         // backward: CTA i warms the L2 with the tiles of CTA i + pf_stride (0 = off)
 };
-
-// keep-bit buffer of the step that is running (double-buffered on the parity of the step counter when `keepbits_alt` is set)
-__device__ __forceinline__ uint32_t* keep_buffer(const AttnParams& p, uint32_t step) {
-    return (p.keepbits_alt != nullptr && (step & 1u)) ? p.keepbits_alt : p.keepbits;
-}
 
 // 2^x as ONE MUFU.EX2.  exp2f() costs four issue slots per value -- compare against -126, pre-scale by 0.5, MUFU, square --
 // to return denormal results; here x <= 0 always and a probability below 2^-126 is 0 in the bf16 P tile anyway.
@@ -213,28 +205,20 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
         const int chunks_per_row = p.S >> 3;
         uint32_t kbits[4] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu};
         if (p.thresh16) {
-            uint32_t* kb = keep_buffer(p, step);
-            // Filled ahead of time (on a background stream, during the previous step) by attn_keepbits_kernel?  Then the 16
-            // Philox blocks per thread -- 56 % of this kernel's instructions -- are four 4-byte loads.  Warp-uniform.
-            const bool pre = p.ready != nullptr && p.ready[step & 1u] == step + 1u;
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
                 const int kc = half * 128 + c * 32;
                 if (qvalid && kc < p.S) {
                     uint32_t bits = 0;
-                    if (pre) {
-                        bits = __ldg(kb + grow * (p.S >> 5) + (kc >> 5));
-                    } else {
 #pragma unroll
-                        for (int g8 = 0; g8 < 4; ++g8) {
-                            const int key0 = kc + g8 * 8;
-                            uint32_t keep = 0xFFu;
-                            if (key0 < p.S)
-                                keep = dropout_keep8(p.seed, p.site, step, (unsigned long long)grow * chunks_per_row + (key0 >> 3), p.thresh16);
-                            bits |= keep << (8 * g8);
-                        }
-                        kb[grow * (p.S >> 5) + (kc >> 5)] = bits;  // reused by the backward kernel
+                    for (int g8 = 0; g8 < 4; ++g8) {
+                        const int key0 = kc + g8 * 8;
+                        uint32_t keep = 0xFFu;
+                        if (key0 < p.S)
+                            keep = dropout_keep8(p.seed, p.site, step, (unsigned long long)grow * chunks_per_row + (key0 >> 3), p.thresh16);
+                        bits |= keep << (8 * g8);
                     }
+                    p.keepbits[grow * (p.S >> 5) + (kc >> 5)] = bits;  // reused by the backward kernel
                     kbits[c] = bits;
                 }
             }
@@ -591,7 +575,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
         float delta0 = 0.f, delta1 = 0.f, L0 = 0.f, L1 = 0.f;
         uint32_t kbits[NKB][2];
         {
-            const uint32_t* kbuf = p.thresh16 ? keep_buffer(p, *p.d_step) : nullptr;  // the buffer the forward of THIS step used
+            const uint32_t* kbuf = p.thresh16 ? p.keepbits : nullptr;
             bool ok[2];
 #pragma unroll
             for (int i = 0; i < 2; ++i) ok[i] = (i < n_qt) && (qbase + i * 128 + row < p.S);
@@ -848,30 +832,6 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
     }
 }
 
-// ================================================================================================ keep bits ahead of time
-// The dropout decisions of the NEXT step's attention probabilities, drawn off the critical path: one thread per 32-key word
-// (four Philox4x32-10 blocks), launched on a low-priority background stream inside the captured step, so that its short
-// CTAs run in the partly idle tails of the GEMM waves and next to the HBM-bound kernels.  Same counters as the forward
-// kernel's own path (and as the unfused softmax kernel): element index = row * S + key, 8 elements per block.
-__global__ void __launch_bounds__(256)
-attn_keepbits_kernel(uint32_t* __restrict__ buf0, uint32_t* __restrict__ buf1, long long n_words, unsigned long long seed,
-                     uint32_t site, const uint32_t* __restrict__ d_step, uint32_t step_offset, uint32_t thresh16) {
-    const uint32_t step = *d_step + step_offset;
-    uint32_t* out = (step & 1u) ? buf1 : buf0;
-    for (long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x; w < n_words; w += (long long)gridDim.x * blockDim.x) {
-        uint32_t bits = 0;
-#pragma unroll
-        for (int g8 = 0; g8 < 4; ++g8)
-            bits |= dropout_keep8(seed, site, step, (unsigned long long)w * 4 + g8, thresh16) << (8 * g8);
-        out[w] = bits;
-    }
-}
-// stream-ordered behind the generator: publishes "buffer (step & 1) holds the bits of `step`"
-__global__ void attn_keepbits_mark_kernel(uint32_t* ready, const uint32_t* d_step, uint32_t step_offset) {
-    const uint32_t step = *d_step + step_offset;
-    ready[step & 1u] = step + 1u;
-}
-
 EncodeTiledFn encode_fn() {
     static EncodeTiledFn fn = nullptr;
     if (!fn) {
@@ -906,8 +866,7 @@ int head_map(CUtensorMap* m, const void* ptr, int B, int S, int slots, int box_r
 }
 
 AttnParams make_params(int B, int S, int nh, float p_drop, uint64_t seed, uint32_t site, const uint32_t* d_step,
-                       const int32_t* mask, float* lse, uint32_t* keepbits, float* gbias = nullptr,
-                       uint32_t* keepbits_alt = nullptr, const uint32_t* ready = nullptr) {
+                       const int32_t* mask, float* lse, uint32_t* keepbits, float* gbias = nullptr) {
     AttnParams p;
     p.B = B; p.S = S; p.nh = nh;
     p.scale = 1.0f / sqrtf((float)DH);
@@ -915,8 +874,6 @@ AttnParams make_params(int B, int S, int nh, float p_drop, uint64_t seed, uint32
     p.inv_keep = p_drop > 0.f ? 1.0f / (1.0f - p_drop) : 1.0f;
     p.seed = seed; p.site = site; p.d_step = d_step; p.mask = mask; p.lse = lse; p.keepbits = keepbits;
     p.gbias = gbias;
-    p.keepbits_alt = keepbits_alt;
-    p.ready = ready;
     p.pf_stride = 0;
     return p;
 }
@@ -926,30 +883,9 @@ AttnParams make_params(int B, int S, int nh, float p_drop, uint64_t seed, uint32
 extern "C" int polus_attention_supported(int S, int dh) { return (dh == DH && S >= 32 && S <= 512 && S % 32 == 0) ? 1 : 0; }
 extern "C" size_t polus_attention_keepbits_words(int B, int S, int nh) { return (size_t)B * nh * S * (S / 32); }
 
-extern "C" int polus_attention_keepbits(uint32_t* keepbits, uint32_t* keepbits_alt, uint32_t* ready, int B, int S, int nh,
-                                        float p_drop, uint64_t seed, uint32_t site, const uint32_t* d_step,
-                                        uint32_t step_offset, void* stream) {
-    POLUS_REQUIRE(keepbits != nullptr && keepbits_alt != nullptr && ready != nullptr && d_step != nullptr,
-                  "polus_attention_keepbits: two buffers, the ready flags and d_step are required");
-    POLUS_REQUIRE(p_drop > 0.f && S % 32 == 0, "polus_attention_keepbits: needs p_drop > 0 and S %% 32 == 0");
-    const long long n_words = (long long)B * nh * S * (S / 32);
-    if (n_words == 0) return 0;
-    const uint32_t thresh16 = (uint32_t)lrintf(p_drop * 65536.0f);
-    const long long blocks = (n_words + 255) / 256;
-    const long long cap = (long long)polus_num_sms() * 64;   // many short CTAs: they only fill gaps
-    attn_keepbits_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, (cudaStream_t)stream>>>(keepbits, keepbits_alt, n_words, seed, site,
-                                                                                             d_step, step_offset, thresh16);
-    g_launch_count++;
-    POLUS_LAUNCH_CHECK();
-    attn_keepbits_mark_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(ready, d_step, step_offset);
-    g_launch_count++;
-    POLUS_LAUNCH_CHECK();
-    return 0;
-}
-
 extern "C" int polus_attention_fwd(const polus_bf16_t* qkv, const int32_t* mask, int B, int S, int nh, int dh, float p_drop,
                                    uint64_t seed, uint32_t site, const uint32_t* d_step, polus_bf16_t* ctx, float* lse,
-                                   uint32_t* keepbits, uint32_t* keepbits_alt, const uint32_t* ready, void* stream) {
+                                   uint32_t* keepbits, void* stream) {
     POLUS_REQUIRE(polus_attention_supported(S, dh), "polus_attention_fwd: needs head_dim 64 and S <= 512, S %% 32 == 0 (got S=%d dh=%d)", S, dh);
     POLUS_REQUIRE(p_drop == 0.f || (d_step != nullptr && keepbits != nullptr), "polus_attention_fwd: dropout needs d_step and keepbits");
     if (B == 0) return 0;
@@ -964,7 +900,7 @@ extern "C" int polus_attention_fwd(const polus_bf16_t* qkv, const int32_t* mask,
         POLUS_CHECK_CUDA(cudaFuncSetAttribute(attn_fwd_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdCfg<4>::SMEM));
         set = true;
     }
-    AttnParams p = make_params(B, S, nh, p_drop, seed, site, d_step, mask, lse, keepbits, nullptr, keepbits_alt, ready);
+    AttnParams p = make_params(B, S, nh, p_drop, seed, site, d_step, mask, lse, keepbits);
     const int q_tiles = (S + 127) / 128;
     if (S <= 256)
         POLUS_CHECK_CUDA(polus_launch_pdl(attn_fwd_kernel<2>, dim3(B * nh * q_tiles), dim3(FwdCfg<2>::THREADS), FwdCfg<2>::SMEM, (cudaStream_t)stream, tq, to, p));
@@ -978,7 +914,7 @@ extern "C" int polus_attention_fwd(const polus_bf16_t* qkv, const int32_t* mask,
 extern "C" int polus_attention_bwd(const polus_bf16_t* qkv, const int32_t* mask, const polus_bf16_t* ctx,
                                    const polus_bf16_t* dctx, const float* lse, int B, int S, int nh, int dh, float p_drop,
                                    uint64_t seed, uint32_t site, const uint32_t* d_step, const uint32_t* keepbits,
-                                   const uint32_t* keepbits_alt, polus_bf16_t* dqkv, float* gbias_qkv, void* stream) {
+                                   polus_bf16_t* dqkv, float* gbias_qkv, void* stream) {
     POLUS_REQUIRE(polus_attention_supported(S, dh), "polus_attention_bwd: needs head_dim 64 and S <= 512, S %% 32 == 0 (got S=%d dh=%d)", S, dh);
     POLUS_REQUIRE(p_drop == 0.f || keepbits != nullptr, "polus_attention_bwd: dropout needs the forward's keepbits");
     if (B == 0) return 0;
@@ -998,8 +934,7 @@ extern "C" int polus_attention_bwd(const polus_bf16_t* qkv, const int32_t* mask,
         set = true;
     }
     POLUS_REQUIRE(p_drop == 0.f || d_step != nullptr, "polus_attention_bwd: dropout needs d_step");
-    AttnParams p = make_params(B, S, nh, p_drop, seed, site, d_step, mask, const_cast<float*>(lse), const_cast<uint32_t*>(keepbits), gbias_qkv,
-                               const_cast<uint32_t*>(keepbits_alt), nullptr);
+    AttnParams p = make_params(B, S, nh, p_drop, seed, site, d_step, mask, const_cast<float*>(lse), const_cast<uint32_t*>(keepbits), gbias_qkv);
     static const int pf_env = getenv("POLUS_ATTN_PREFETCH") ? atoi(getenv("POLUS_ATTN_PREFETCH")) : 1;
     p.pf_stride = pf_env > 0 ? pf_env * polus_num_sms() : 0;   // CTA i warms the L2 for CTA i + (number of SMs): one wave ahead
     const int n_half = (S + 255) / 256;

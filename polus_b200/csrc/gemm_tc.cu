@@ -28,7 +28,6 @@
 #include "ptx.cuh"
 #include <cuda.h>
 #include <atomic>
-#include <stdlib.h>
 
 extern std::atomic<long long> g_launch_count;
 
@@ -46,6 +45,7 @@ constexpr int STG_BLOCK = 32 * 128;                       // one staging block: 
 constexpr int kSmemTotal = 227 * 1024;
 constexpr int kBarBytes = 512;
 constexpr int kMaxStages = 8;
+constexpr int kGroupM = 8;  // m-tiles per rasterisation group (TcParams::group_m)
 
 struct TcParams {
     int M, N, K;
@@ -66,17 +66,16 @@ struct TcParams {
     int c2_grad;      // C2 = act'(pre-activation) instead of the pre-activation
     int has_emul;     // C = (alpha A.B^T + bias) * Emul, Emul read through tmC2
     float* colsum;    // colsum[n] += sum_m C[m,n]
-    int l2_hint;      // L2 evict_first hints: 1 = C2 stores, 2 = C stores, 4 = multiplier-tile loads
     int c2_u8;        // C2 (forward) / Emul (backward) holds gelu' as 8-bit fixed point (common.cuh d8_pack4): 16-warp kernel only
 };
 
 template <int BN, int CG>
 struct Cfg {
+    static_assert(BN == 64 || BN == 128 || BN == 256, "tile widths: 64, 128, 256");
+    static_assert(CG == 1 || (CG == 2 && BN >= 128), "one CTA, or a pair that splits the B tile into 64-column multiples");
     static constexpr int BN_LOCAL = BN / CG;  // rows of the B tile this CTA stages
-    // MN-major B arrives in 64-column groups (one 128-byte swizzle atom wide): a 96-column share (BN = 192 on a pair)
-    // fetches two full groups and the MMA reads the first 96 columns; the slot size is the same for both majors
-    static constexpr int B_GROUPS = (BN_LOCAL + 63) / 64;
-    static constexpr int B_STAGE_BYTES = (BN_LOCAL < 64 ? BN_LOCAL : B_GROUPS * 64) * BK * 2;
+    static constexpr int B_GROUPS = BN_LOCAL / 64;  // MN-major B arrives in 64-column groups (one 128-byte swizzle atom wide)
+    static constexpr int B_STAGE_BYTES = BN_LOCAL * BK * 2;
     static constexpr int kStageBytes = A_STAGE_BYTES + B_STAGE_BYTES;
     static constexpr int kTmemCols = 2 * BN <= 32 ? 32 : (2 * BN <= 64 ? 64 : (2 * BN <= 128 ? 128 : (2 * BN <= 256 ? 256 : 512)));
     static int stages(int stg_warp) {
@@ -86,7 +85,7 @@ struct Cfg {
     static int smem_bytes(int stg_warp) { return 1024 + stages(stg_warp) * kStageBytes + kEpiWarps * stg_warp + kBarBytes; }
     static constexpr int kColBlocks = BN / 64;                       // 64-column blocks per tile
     static constexpr int kEpiActive = kColBlocks >= 2 ? 8 : 4;        // epilogue warps that do work
-    static constexpr int kBlocksPerWarp = kColBlocks >= 2 ? (kColBlocks + 1) / 2 : 1;  // (BN = 192: 2 + 1 blocks)
+    static constexpr int kBlocksPerWarp = kColBlocks >= 2 ? kColBlocks / 2 : 1;
 };
 
 __device__ __forceinline__ void red_add_v2(float* addr, float a, float b) {
@@ -187,11 +186,7 @@ __device__ __forceinline__ void stage_row_f32(uint8_t* block, int lane, const fl
     }
 }
 
-// CL = CTAs per cluster: CG, or 4 (two CTA pairs stacked along M that compute the tiles (2mt, nt) and (2mt+1, nt) and SHARE
-// the B tile: each of the four CTAs fetches half of its pair's share and multicasts it to its counterpart in the other
-// pair, so a k-block costs every CTA 24 KB of L2 reads instead of 32 KB -- the 256x256 pair tile at ~1200 TFLOP/s reads
-// ~9.5 TB/s from L2, against a measured chip limit of ~6300 B/clk, B300_MICROARCH).
-template <int BN, bool A_MN, bool B_MN, int CG, int EPI, int CL>
+template <int BN, bool A_MN, bool B_MN, int CG, int EPI>
 __global__ void __launch_bounds__(128 + 32 * EPI, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmC2, const TcParams p) {
@@ -199,16 +194,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int kStages = p.n_stages;
     constexpr int BN_LOCAL = C::BN_LOCAL;
     constexpr int B_STAGE_BYTES = C::B_STAGE_BYTES;
-    // bytes landing on the leader's barrier per k-block (K-major B boxes hold exactly BN_LOCAL rows)
-    constexpr uint32_t kStageTx = (A_STAGE_BYTES + (B_MN ? B_STAGE_BYTES : BN_LOCAL * BK * 2)) * CG;
-    static_assert(CL == CG || (CL == 4 && CG == 2), "cluster is one CTA, one pair, or two pairs");
-    constexpr int PP = CL / CG;  // CTA pairs (or single CTAs) per cluster
-    const uint32_t cluster_rank = CL > 1 ? ptx::cluster_ctarank() : 0u;
-    const uint32_t cta_rank = CG == 2 ? (cluster_rank & 1u) : 0u;  // position inside the pair
-    const int cpair = CG == 2 ? (int)(cluster_rank >> 1) : 0;  // which CTA pair of the cluster
+    constexpr uint32_t kStageTx = C::kStageBytes * CG;  // bytes landing on the leader's barrier per k-block
+    const uint32_t cta_rank = CG == 2 ? ptx::cluster_ctarank() : 0u;  // position inside the pair
     const bool is_leader = cta_rank == 0;
-    const int tile0 = (int)(blockIdx.x / CL);
-    const int tile_step = (int)(gridDim.x / CL);
+    const int tile0 = (int)(blockIdx.x / CG);
+    const int tile_step = (int)(gridDim.x / CG);
 
     // 1024-byte alignment (128B-swizzle atoms) comes from the declaration, which also keeps the pointer in the shared
     // address space for the compiler (LDS / STS instead of generic LD / ST in the staging code)
@@ -237,7 +227,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (warp == 1 && lane == 0) {
         for (int s = 0; s < kStages; ++s) {
             ptx::mbar_init(&full_bar[s], 1);
-            ptx::mbar_init(&empty_bar[s], PP);  // one commit per pair whose tensor cores read (a multicast copy of) this slot
+            ptx::mbar_init(&empty_bar[s], 1);
         }
         for (int s = 0; s < 2; ++s) {
             ptx::mbar_init(&tfull_bar[s], 1);
@@ -252,7 +242,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     }
     ptx::tc_fence_before();
     __syncthreads();
-    if (CL > 1) ptx::cluster_sync();  // peer barriers initialised before any remote arrive / multicast commit
+    if (CG > 1) ptx::cluster_sync();  // peer barriers initialised before any remote arrive / multicast commit
     ptx::tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     pdl_wait();  // operands / outputs of earlier kernels are touched only from here on
@@ -265,7 +255,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int g = r / per_group;
         const int gm = min(p.group_m, p.m_tiles - g * p.group_m);  // the last group may be narrower
         const int rr = r - g * per_group;
-        mt = (g * p.group_m + rr % gm) * PP + cpair;  // m_tiles counts cluster rows; this pair's 256-row tile inside it
+        mt = g * p.group_m + rr % gm;
         nt = rr / gm;
         sp = t % p.split_k;
         t /= p.split_k;
@@ -301,13 +291,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         for (int g = 0; g < BM / 64; ++g)
                             load(a + g * (BK * 128), &tmA, &full_bar[stage], m0 + g * 64, kb * BK, b0, b1);
                     }
-                    if (CL == 4) {
-                        // half of this CTA's B share (64 of its 128 tile columns), multicast to the same position of
-                        // the other pair; the other half arrives from there
-                        const uint16_t mask = (uint16_t)((1u << cta_rank) | (1u << (cta_rank + 2)));
-                        if (!B_MN) ptx::tma_load_4d_2sm_mc(b + cpair * 8192, &tmB, &full_bar[stage], mask, kb * BK, n0 + cpair * 64, b0, b1);
-                        else ptx::tma_load_4d_2sm_mc(b + cpair * (BK * 128), &tmB, &full_bar[stage], mask, n0 + cpair * 64, kb * BK, b0, b1);
-                    } else if (!B_MN) {
+                    if (!B_MN) {
                         load(b, &tmB, &full_bar[stage], kb * BK, n0, b0, b1);
                     } else {
 #pragma unroll
@@ -355,7 +339,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         else ptx::umma_bf16(tmem_d, ad, bd, idesc, accum);
                     }
                     // smem slot reusable (in both CTAs of the pair) once these MMAs retire
-                    if (CG == 2) ptx::umma_commit_2sm(&empty_bar[stage], (uint16_t)((1u << CL) - 1u));
+                    if (CG == 2) ptx::umma_commit_2sm(&empty_bar[stage]);
                     else ptx::umma_commit(&empty_bar[stage]);
                     if (++stage == kStages) {
                         stage = 0;
@@ -363,7 +347,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     }
                 }
                 // accumulator complete -> epilogue warps of both CTAs
-                if (CG == 2) ptx::umma_commit_2sm(&tfull_bar[acc], (uint16_t)(3u << (2 * cpair)));
+                if (CG == 2) ptx::umma_commit_2sm(&tfull_bar[acc]);
                 else ptx::umma_commit(&tfull_bar[acc]);
                 if (++acc == 2) {
                     acc = 0;
@@ -382,7 +366,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int e = warp - 4;
         const int quad = e & 3;
         const int csub = e >> 2;
-        const uint64_t pol_ef = ptx::l2_policy_evict_first();
         constexpr int kCPW = (BN / 32) / 4 > 0 ? (BN / 32) / 4 : 1;  // 32-column chunks per warp per tile
         const uint32_t sC = ptx::smem_u32(sStage) + (uint32_t)e * 4096u;  // [32 rows][64 B] C
         const uint32_t sX = sC + 2048u;                                    // [32 rows][64 B] C2 or multiplier
@@ -414,19 +397,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 uint64_t* ebar = &emul_bar[buf * 16 + e];
                 const uint32_t dstX = sX + (uint32_t)buf * 1024u;
                 ptx::mbar_expect_tx(ebar, p.c2_u8 ? 1024 : 2048);   // 32 x 32 multipliers, bf16 or 8-bit
-                if (p.l2_hint & 4) {   // read once, by this warp: evict first
-                    asm volatile(
-                        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-                        ::"r"(dstX), "l"(reinterpret_cast<uint64_t>(&tmC2)), "r"(ptx::smem_u32(ebar)),
-                        "r"(nt * BN + (csub * kCPW + i) * 32), "r"((mt * CG + (int)cta_rank) * BM + quad * 32), "r"(b0), "r"(b1), "l"(pol_ef)
-                        : "memory");
-                } else {
-                    asm volatile(
-                        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-                        ::"r"(dstX), "l"(reinterpret_cast<uint64_t>(&tmC2)), "r"(ptx::smem_u32(ebar)),
-                        "r"(nt * BN + (csub * kCPW + i) * 32), "r"((mt * CG + (int)cta_rank) * BM + quad * 32), "r"(b0), "r"(b1)
-                        : "memory");
-                }
+                asm volatile(
+                    "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
+                    ::"r"(dstX), "l"(reinterpret_cast<uint64_t>(&tmC2)), "r"(ptx::smem_u32(ebar)),
+                    "r"(nt * BN + (csub * kCPW + i) * 32), "r"((mt * CG + (int)cta_rank) * BM + quad * 32), "r"(b0), "r"(b1)
+                    : "memory");
             }
         };
         auto sts16 = [&](uint32_t tile, int chunk, const float* v8) {  // 8 values -> 16-byte chunk `chunk` of row `lane`
@@ -435,13 +410,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(tile + (uint32_t)lane * 64u + (((uint32_t)chunk ^ swz) << 4)),
                          "r"(u[0]), "r"(u[1]), "r"(u[2]), "r"(u[3]) : "memory");
         };
-        auto tma_store32 = [&](const CUtensorMap* map, uint32_t tile, int c0, int c1, int c2, int c3, bool evict_first) {
-            if (evict_first)
-                asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3, %4, %5}], [%1], %6;"
-                             ::"l"(reinterpret_cast<uint64_t>(map)), "r"(tile), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "l"(pol_ef) : "memory");
-            else
-                asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-                             ::"l"(reinterpret_cast<uint64_t>(map)), "r"(tile), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
+        auto tma_store32 = [&](const CUtensorMap* map, uint32_t tile, int c0, int c1, int c2, int c3) {
+            asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
+                         ::"l"(reinterpret_cast<uint64_t>(map)), "r"(tile), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
         };
         int pf_t = tile0, pf_i = -1;
         if (p.has_emul) {
@@ -584,8 +555,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 ptx::fence_proxy_async_smem();
                 __syncwarp();
                 if (lane == 0) {
-                    tma_store32(&tmC, sC, col0, row0, b0, b1, (p.l2_hint & 2) != 0);  // rows >= M / columns >= N are clipped by the tensor map
-                    if (p.has_c2) tma_store32(&tmC2, sX, col0, row0, b0, b1, (p.l2_hint & 1) != 0);
+                    tma_store32(&tmC, sC, col0, row0, b0, b1);  // rows >= M / columns >= N are clipped by the tensor map
+                    if (p.has_c2) tma_store32(&tmC2, sX, col0, row0, b0, b1);
                     ptx::tma_store_commit();
                 }
                 store_pending = true;
@@ -607,7 +578,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             ptx::tc_fence_before();
             __syncwarp();
             if (lane == 0) {
-                if (CG == 2) ptx::mbar_arrive_remote(&tempty_bar[acc], 2 * cpair);
+                if (CG == 2) ptx::mbar_arrive_remote(&tempty_bar[acc], 0);
                 else ptx::mbar_arrive(&tempty_bar[acc]);
             }
             if (++acc == 2) {
@@ -778,7 +749,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             ptx::tc_fence_before();
             __syncwarp();
             if (lane == 0) {
-                if (CG == 2) ptx::mbar_arrive_remote(&tempty_bar[acc], 2 * cpair);  // the pair leader's MMA thread waits on it
+                if (CG == 2) ptx::mbar_arrive_remote(&tempty_bar[acc], 0);  // the pair leader's MMA thread waits on it
                 else ptx::mbar_arrive(&tempty_bar[acc]);
             }
             if (++acc == 2) {
@@ -791,7 +762,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 
     ptx::tc_fence_before();
     __syncthreads();
-    if (CL > 1) ptx::cluster_sync();  // the peers may still be reading our smem / arriving on our barriers
+    if (CG > 1) ptx::cluster_sync();  // the peer may still be reading our smem / arriving on our barriers
     if (warp == 2) {
         ptx::tc_fence_after();
         if (CG == 2) ptx::tmem_dealloc_2sm<C::kTmemCols>(tmem_base);
@@ -851,10 +822,10 @@ int make_map(CUtensorMap* map, const polus_operand_t& op, long long mn_len, long
     return encode_map(map, op.ptr, inner, rows, op.ld, batch0, op.bs0, batch1, op.bs1, op.mn_major ? BK : box_mn);
 }
 
-template <int BN, bool A_MN, bool B_MN, int CG, int EPI = 8, int CL = CG>
+template <int BN, bool A_MN, bool B_MN, int CG, int EPI = 8>
 int launch(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const CUtensorMap& tc2,
            const TcParams& p_in, cudaStream_t st) {
-    auto kern = gemm_tc_kernel<BN, A_MN, B_MN, CG, EPI, CL>;
+    auto kern = gemm_tc_kernel<BN, A_MN, B_MN, CG, EPI>;
     using C = Cfg<BN, CG>;
     static bool attr_set = false;
     if (!attr_set) {
@@ -870,28 +841,12 @@ int launch(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, 
     cfg.stream = st;
     cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CL;
+    attr[0].val.clusterDim.x = CG;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
-    int groups = polus_num_sms() / CL;
-    if (CL == 4) {
-        // four-CTA clusters must sit inside one GPC: not every SM can be part of one, and the persistent tile loop
-        // needs all its clusters resident at once
-        static int max_clusters = 0;
-        if (max_clusters == 0) {
-            cfg.gridDim = dim3(groups * CL);
-            cfg.attrs = attr;
-            cfg.numAttrs = 1;
-            int n = 0;
-            if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) == cudaSuccess && n > 0) max_clusters = n;
-            else max_clusters = groups;
-            cudaGetLastError();
-            if (getenv("POLUS_GEMM_DEBUG")) fprintf(stderr, "[polus_gemm_tc] 4-CTA clusters resident: %d (of %d wanted)\n", max_clusters, groups);
-        }
-        if (max_clusters < groups) groups = max_clusters;
-    }
+    int groups = polus_num_sms() / CG;
     if (p.num_tiles < groups) groups = p.num_tiles;
-    cfg.gridDim = dim3(groups * CL);
+    cfg.gridDim = dim3(groups * CG);
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
@@ -912,6 +867,56 @@ int launch_major(int a_mn, int b_mn, const CUtensorMap& ta, const CUtensorMap& t
 }
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+struct TilePlan {
+    int CG;      // CTAs per tile: 2 = a CTA pair on a 256-row tile, 1 = one CTA on a 128-row tile
+    int BN;      // tile width: 64, 128 or 256
+    int split;   // K splits (before clamping to the number of k-blocks)
+    bool epi16;  // 16-epilogue-warp kernel
+};
+
+// The one place that picks the kernel for a problem: the dispatch in polus_gemm_tc launches what this returns, and
+// why_unsupported accepts the 8-bit derivative only where it returns the 16-warp kernel.
+TilePlan plan_tiles(const polus_gemm_t* g, int sms) {
+    const int batch0 = g->batch0 < 1 ? 1 : g->batch0;
+    const int batch1 = g->batch1 < 1 ? 1 : g->batch1;
+    TilePlan t;
+    // CTA pairs (cta_group::2, 256-row tiles) whenever there are at least two 128-row tiles to pair up
+    t.CG = (g->M > BM && g->N > 64) ? 2 : 1;
+    const long long mt = cdiv(g->M, BM * t.CG);
+    const long long nb = (long long)batch0 * batch1;
+    const int kb_total = cdiv(g->K, BK);
+    const long long groups = sms / t.CG;
+    // Tile width and split-K.
+    //  * accumulate GEMMs with split_k == 0 (wgrad: few output tiles, very long K): 256-wide tiles whenever N allows
+    //    (a 128-wide pair tile needs 96 B/clk/SM of operand traffic, more than L2 delivers) and the split that
+    //    minimises waves x (k-blocks per split + fixed tile overhead).
+    //  * everything else: the widest tile that still yields one full wave of CTAs.
+    const bool wgrad = g->split_k == 0 && g->accumulate && g->act == POLUS_ACT_NONE && g->C2 == nullptr;
+    t.split = g->split_k < 1 ? 1 : g->split_k;
+    if (g->N <= 64) t.BN = 64;
+    else if (g->N <= 128) t.BN = 128;
+    else if (wgrad) t.BN = 256;
+    else t.BN = mt * cdiv(g->N, 256) * nb * t.split * t.CG >= sms ? 256 : 128;
+    if (wgrad) {
+        const long long tiles = mt * cdiv(g->N, t.BN) * nb;
+        const int max_split = kb_total / 4 > 1 ? kb_total / 4 : 1;  // >= 4 k-blocks per split
+        long long best_cost = -1;
+        for (int sp = 1; sp <= max_split && sp <= 32; ++sp) {
+            const long long waves = (tiles * sp + groups - 1) / groups;
+            const long long cost = waves * (cdiv(kb_total, sp) + 8);
+            if (best_cost < 0 || cost < best_cost) {
+                best_cost = cost;
+                t.split = sp;
+            }
+        }
+    }
+    // epilogues with per-element math run on the 16-epilogue-warp instantiation (256-wide pair tiles, A K-major:
+    // the FFN-up forward GEMM and the dgrad GEMM that applies act' and sums the bias gradient)
+    t.epi16 = t.CG == 2 && t.BN == 256 && g->c_dtype != POLUS_F32 && !g->A.mn_major &&
+              (g->act != POLUS_ACT_NONE || g->Emul != nullptr || g->C2 != nullptr);
+    return t;
+}
 
 const char* why_unsupported(const polus_gemm_t* g) {
     if (g->A.dtype != POLUS_BF16 || g->B.dtype != POLUS_BF16) return "operands must be bf16";
@@ -934,14 +939,10 @@ const char* why_unsupported(const polus_gemm_t* g) {
     if (g->c2_kind < 0 || g->c2_kind > 2) return "c2_kind";
     if (g->c2_kind == 2) {
         // 8-bit gelu' (C2 of a GELU forward, or the Emul tile of the dgrad that consumes it): only the 16-epilogue-warp
-        // kernel on 256-wide pair tiles implements it -- the same conditions as the dispatch in polus_gemm_tc
-        static const int epi_env = getenv("POLUS_GEMM_EPI16") ? atoi(getenv("POLUS_GEMM_EPI16")) : 1;
-        static const int cg_env = getenv("POLUS_GEMM_CG") ? atoi(getenv("POLUS_GEMM_CG")) : 0;
-        const int b0 = g->batch0 < 1 ? 1 : g->batch0, b1 = g->batch1 < 1 ? 1 : g->batch1;
-        if (!epi_env || cg_env == 1) return "8-bit derivative needs the 16-warp pair kernel";
+        // kernel implements it
         if (!(g->C2 != nullptr && g->act == POLUS_ACT_GELU) && g->Emul == nullptr) return "8-bit derivative: GELU forward with C2, or Emul";
-        if (g->c_dtype != POLUS_BF16 || g->A.mn_major || g->M <= BM || g->N <= 128 || g->N % 32) return "8-bit derivative: shape";
-        if ((long long)cdiv(g->M, 2 * BM) * cdiv(g->N, 256) * b0 * b1 * 2 < polus_num_sms()) return "8-bit derivative: needs 256-wide tiles";
+        if (!plan_tiles(g, polus_num_sms()).epi16) return "8-bit derivative needs the 16-warp pair kernel";
+        if (g->N % 32) return "8-bit derivative: N must be a multiple of 32";
         if (g->ldc % 16 || g->cbs0 % 16 || g->cbs1 % 16) return "8-bit derivative: strides must be multiples of 16";
     }
     return nullptr;
@@ -956,82 +957,27 @@ extern "C" int polus_gemm_tc(const polus_gemm_t* g, void* stream) {
     POLUS_REQUIRE(why == nullptr, "polus_gemm_tc: unsupported problem (%s) M=%d N=%d K=%d", why, g->M, g->N, g->K);
     const int batch0 = g->batch0 < 1 ? 1 : g->batch0;
     const int batch1 = g->batch1 < 1 ? 1 : g->batch1;
-    const int sms = polus_num_sms();
-
-    // CTA pairs (cta_group::2, 256-row tiles) whenever there are at least two 128-row tiles to pair up
-    static const int cg_env = getenv("POLUS_GEMM_CG") ? atoi(getenv("POLUS_GEMM_CG")) : 0;
-    const int CG = (g->M > BM && g->N > 64 && cg_env != 1) ? 2 : 1;
+    const TilePlan plan = plan_tiles(g, polus_num_sms());
+    const int CG = plan.CG, BN = plan.BN;
     const long long mt = cdiv(g->M, BM * CG);
     const long long nb = (long long)batch0 * batch1;
-    const int kb_total = cdiv(g->K, BK);
-    // Tile width and split-K.
-    //  * accumulate GEMMs with split_k == 0 (wgrad: few output tiles, very long K): 256-wide tiles whenever N allows
-    //    (a 128-wide pair tile needs 96 B/clk/SM of operand traffic, more than L2 delivers) and the split that
-    //    minimises waves x (k-blocks per split + fixed tile overhead).
-    //  * everything else: the widest tile that still yields one full wave of CTAs.
-    int split = g->split_k < 1 ? 1 : g->split_k;
-    int BN;
-    const long long groups = sms / CG;
-    if (g->N <= 64) BN = 64;
-    else if (g->N <= 128) BN = 128;
-    else if (g->split_k == 0 && g->accumulate && g->act == POLUS_ACT_NONE && g->C2 == nullptr) BN = 256;
-    else {
-        const long long ctas256 = mt * cdiv(g->N, 256) * nb * split * CG;
-        BN = ctas256 >= sms ? 256 : 128;
-        // 192-wide pair tiles (POLUS_GEMM_BN192=1, off by default): N = 768 outputs at 32768 rows are 384 tiles of 256 columns
-        // = 5.2 waves on 74 pairs, but 512 tiles of 192 = 6.9 waves.  MEASURED SLOWER (batch 128: fwd_ffn2 100.5 -> 114.3 us,
-        // dgrad_ffn1 99.9 -> 113.1, dgrad_qkv 78.2 -> 88.1, profiles/r01_gemm_shapes_v17_b128_bn{256,192}.log): the A tile is
-        // reused over 192 instead of 256 columns and the pair becomes operand-bandwidth bound, which costs more than the
-        // partly filled sixth wave.  Kept as a tested instantiation for shapes / parts where the balance differs.
-        const char* bn192_s = getenv("POLUS_GEMM_BN192");
-        const int bn192_env = bn192_s ? atoi(bn192_s) : 0;
-        const bool plain_epi = g->act == POLUS_ACT_NONE && g->C2 == nullptr && g->Emul == nullptr;
-        if (bn192_env && BN == 256 && CG == 2 && plain_epi && g->N % 192 == 0) {
-            const long long w256 = cdiv(mt * cdiv(g->N, 256) * nb * split, groups) * 256;
-            const long long w192 = cdiv(mt * cdiv(g->N, 192) * nb * split, groups) * 192;
-            if (w192 * 100 <= w256 * 95) BN = 192;
-        }
-    }
-    if (g->split_k == 0 && g->accumulate && g->act == POLUS_ACT_NONE && g->C2 == nullptr) {
-        const long long tiles = mt * cdiv(g->N, BN) * nb;
-        const int max_split = kb_total / 4 > 1 ? kb_total / 4 : 1;  // >= 4 k-blocks per split
-        long long best_cost = -1;
-        for (int sp = 1; sp <= max_split && sp <= 32; ++sp) {
-            const long long waves = (tiles * sp + groups - 1) / groups;
-            const long long cost = waves * (cdiv(kb_total, sp) + 8);
-            if (best_cost < 0 || cost < best_cost) {
-                best_cost = cost;
-                split = sp;
-            }
-        }
-    }
-
-    // two-pair clusters sharing the B tile (see the kernel template): plain bf16-output GEMMs on 256-wide pair tiles
-    // with an even number of 256-row tiles.  EXPERIMENT, off by default (POLUS_GEMM_CL4=1): per SM it is ~12 % faster on
-    // the K-major-B shapes, but only 33 four-CTA clusters are resident on this part (132 of 148 SMs), so the launch as a
-    // whole ties (fwd_ffn2 54.2 vs 54.3 us, dgrad_ffn1 52.9 vs 53.1) and loses with MN-major B (fwd_qkv 56 vs 47 us).
-    // Worth it only together with a second kernel on the 16 SMs no cluster can use.
-    static const int cl4_env = getenv("POLUS_GEMM_CL4") ? atoi(getenv("POLUS_GEMM_CL4")) : 0;
-    const bool plain = g->c_dtype == POLUS_BF16 && g->act == POLUS_ACT_NONE && !g->C2 && !g->Emul;
-    const bool cl4 = cl4_env && CG == 2 && BN == 256 && plain && !g->A.mn_major && !g->B.mn_major && mt % 2 == 0 && split == 1;
-    const long long mt_cluster = cl4 ? mt / 2 : mt;
+    int split = plan.split;
 
     TcParams p;
     p.M = g->M;
     p.N = g->N;
     p.K = g->K;
     p.batch0 = batch0;
-    p.m_tiles = (int)mt_cluster;
+    p.m_tiles = (int)mt;
     p.n_tiles = cdiv(g->N, BN);
-    p.kb_total = kb_total;
+    p.kb_total = cdiv(g->K, BK);
     if (split > p.kb_total) split = p.kb_total;
     p.kb_per_split = cdiv(p.kb_total, split);
     p.split_k = cdiv(p.kb_total, p.kb_per_split);
-    p.num_tiles = (int)(mt_cluster * p.n_tiles * p.split_k * nb);
+    p.num_tiles = (int)(mt * p.n_tiles * p.split_k * nb);
     // Rasterisation: concurrently running tiles form (about) an 8 x 9 patch of the tile grid instead of a 74 x 1 column
     // strip, so each A row block and each B column block in flight is shared by 8-9 clusters (measured 1.05-1.15x).
-    static const int group_env = getenv("POLUS_GEMM_GROUP_M") ? atoi(getenv("POLUS_GEMM_GROUP_M")) : 8;
-    p.group_m = (group_env > 0 && group_env < p.m_tiles) ? group_env : p.m_tiles;
+    p.group_m = kGroupM < p.m_tiles ? kGroupM : p.m_tiles;
     p.C = g->C;
     p.ldc = g->ldc;
     p.cbs0 = g->cbs0;
@@ -1045,8 +991,6 @@ extern "C" int polus_gemm_tc(const polus_gemm_t* g, void* stream) {
     p.c2_grad = g->c2_kind >= 1;
     p.has_emul = g->Emul != nullptr;
     p.colsum = g->colsum;
-    static const int l2_env = getenv("POLUS_GEMM_L2HINT") ? atoi(getenv("POLUS_GEMM_L2HINT")) : 0;
-    p.l2_hint = l2_env;
     p.c2_u8 = g->c2_kind == 2;
     p.stg_warp = (p.c_f32 || p.has_c2 || p.has_emul) ? 2 * STG_BLOCK : STG_BLOCK;
     p.n_stages = 0;  // set per instantiation in launch()
@@ -1054,7 +998,7 @@ extern "C" int polus_gemm_tc(const polus_gemm_t* g, void* stream) {
     CUtensorMap ta, tb, tc, tc2;
     int rc = make_map(&ta, g->A, g->M, g->K, batch0, batch1, BM);
     if (rc) return rc;
-    rc = make_map(&tb, g->B, g->N, g->K, batch0, batch1, cl4 ? BN / CG / 2 : BN / CG);
+    rc = make_map(&tb, g->B, g->N, g->K, batch0, batch1, BN / CG);
     if (rc) return rc;
     if (!p.c_f32) {  // bf16 outputs leave through TMA stores of 32-row x 64-column blocks
         rc = encode_map(&tc, g->C, g->N, g->M, g->ldc, batch0, g->cbs0, batch1, g->cbs1, 32);
@@ -1071,10 +1015,7 @@ extern "C" int polus_gemm_tc(const polus_gemm_t* g, void* stream) {
         tc2 = tc;
     }
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    // epilogues with per-element math run on the 16-epilogue-warp instantiation (256-wide pair tiles, A K-major:
-    // the FFN-up forward GEMM and the dgrad GEMM that applies act' and sums the bias gradient)
-    static const int epi_env = getenv("POLUS_GEMM_EPI16") ? atoi(getenv("POLUS_GEMM_EPI16")) : 1;
-    if (CG == 2 && BN == 256 && !p.c_f32 && !g->A.mn_major && epi_env && (p.act != POLUS_ACT_NONE || p.has_emul || p.has_c2)) {
+    if (plan.epi16) {
         // 16 warps x (2 KB C + 2 KB C2 / multiplier), 32 x 32 TMA boxes with the 64-byte swizzle
         p.stg_warp = 2 * STG_BLOCK;
         rc = encode_map(&tc, g->C, g->N, g->M, g->ldc, batch0, g->cbs0, batch1, g->cbs1, 32, 2, 64);
@@ -1089,14 +1030,8 @@ extern "C" int polus_gemm_tc(const polus_gemm_t* g, void* stream) {
         if (g->B.mn_major) return launch<256, false, true, 2, 16>(ta, tb, tc, tc2, p, st);
         return launch<256, false, false, 2, 16>(ta, tb, tc, tc2, p, st);
     }
-    POLUS_REQUIRE(!p.c2_u8, "polus_gemm_tc: the 8-bit derivative needs the 16-warp pair kernel (M=%d N=%d K=%d)", g->M, g->N, g->K);
-    if (cl4) {
-        if (g->B.mn_major) return launch<256, false, true, 2, 8, 4>(ta, tb, tc, tc2, p, st);
-        return launch<256, false, false, 2, 8, 4>(ta, tb, tc, tc2, p, st);
-    }
     if (CG == 2) {
         if (BN == 128) return launch_major<128, 2>(g->A.mn_major, g->B.mn_major, ta, tb, tc, tc2, p, st);
-        if (BN == 192) return launch_major<192, 2>(g->A.mn_major, g->B.mn_major, ta, tb, tc, tc2, p, st);
         return launch_major<256, 2>(g->A.mn_major, g->B.mn_major, ta, tb, tc, tc2, p, st);
     }
     if (BN == 64) return launch_major<64, 1>(g->A.mn_major, g->B.mn_major, ta, tb, tc, tc2, p, st);

@@ -83,45 +83,11 @@ __device__ __forceinline__ void bulk_load(void* smem_dst, const void* gmem_src, 
                  : "memory");
 }
 
-// 2-CTA + multicast: the box lands at the same CTA-relative offset in every CTA of `cta_mask`; each destination's bytes
-// complete on the barrier (same offset) of that destination's pair leader.
-__device__ __forceinline__ void tma_load_4d_2sm_mc(void* smem_dst, const CUtensorMap* map, uint64_t* bar, uint16_t cta_mask,
-                                                   int c0, int c1, int c2, int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-        " [%0], [%1, {%4, %5, %6, %7}], [%2], %3;"
-        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "h"(cta_mask),
-        "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-
 // TMA store: swizzled smem block -> global (rows/columns outside the tensor map are clipped)
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, const void* smem_src, int c0, int c1, int c2, int c3) {
     asm volatile(
         "cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
         ::"l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-// L2 eviction-priority hints (createpolicy): a tensor written for a much later reader -- or read exactly once -- should
-// not push the GEMM's own operands out of the 126 MB L2
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-    uint64_t pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-__device__ __forceinline__ void tma_store_4d_hint(const CUtensorMap* map, const void* smem_src, int c0, int c1, int c2, int c3, uint64_t pol) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3, %4, %5}], [%1], %6;"
-        ::"l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "l"(pol)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_hint(void* smem_dst, const CUtensorMap* map, uint64_t* bar,
-                                                 int c0, int c1, int c2, int c3, uint64_t pol) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint"
-        " [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)),
-        "r"(c0), "r"(c1), "r"(c2), "r"(c3), "l"(pol)
         : "memory");
 }
 // TMA prefetch of one box into L2 (no shared-memory destination, no barrier): warms the L2 for a load that a LATER CTA will issue

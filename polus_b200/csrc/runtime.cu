@@ -41,7 +41,7 @@ bool polus_pdl_enabled() {
 extern "C" {
 
 const char* polus_last_error(void) { return g_err; }
-int polus_version(void) { return 100; }
+int polus_version(void) { return 101; }
 
 int polus_device_count(int* n) {
     POLUS_CHECK_CUDA(cudaGetDeviceCount(n));

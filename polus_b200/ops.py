@@ -48,8 +48,6 @@ def step_counter():
 
 def set_step(value):
     device.upload(step_counter(), np.array([value, 0, 0, 0], np.uint32))
-    if _keep_state:
-        invalidate_keep_state()
 
 
 class Node:
@@ -170,7 +168,6 @@ def run_backward(nodes, loss, before_node=None):
             else:
                 grads[id(t)] = [prev, gi]
     side_join()  # weight gradients issued on the background stream are complete from here on
-    rng_stream_join()  # ... and the next step's dropout bits were drawn from the CURRENT step counter: before the optimizer bumps it
     return grads
 
 
@@ -255,7 +252,6 @@ def side_reset():
     _side["next"] = 0
     _side["dirty"] = False
     _side["opt_dirty"] = False
-    _side["rng_dirty"] = False
 
 
 def side_fork():
@@ -417,12 +413,6 @@ def _gemm_tc_supported(M, N, K, A, B, c_ptr, ldc, c_dtype, **kw):
     return _lib.call("polus_gemm_tc_supported", C.byref(g)) == 1
 
 
-# gelu' stored as 8-bit fixed point by the FFN-up GEMM and read back by the dgrad GEMM of the next layer (c2_kind = 2):
-# both are bound by SM store bandwidth / multiplier-tile traffic, and a byte per element carries the same aggregate
-# gradient error as bf16 (DESIGN.md section 8).  POLUS_GELU_D8=0 keeps the bf16 copy.
-GELU_D8 = _os.environ.get("POLUS_GELU_D8", "1") != "0"
-
-
 def _act_code(act):
     if callable(act):
         act = getattr(act, "__name__", None)
@@ -448,11 +438,14 @@ def linear(x, W, b=None, activation=None, out_dtype=None, defer_bias_grad=False)
         y = Tensor(lead + (N,), BF16)
         # with an activation the GEMM epilogue also stores act'(z) (not z): backward is then one multiply, which the
         # dgrad GEMM of the layer that consumes y applies in its own epilogue together with the bias-gradient column
-        # sums (FUSE_ACT_BWD) -- no pass over the [M,N] tensor for GeluGrad / BiasAddGrad
+        # sums (FUSE_ACT_BWD) -- no pass over the [M,N] tensor for GeluGrad / BiasAddGrad.  GELU's derivative goes as 8-bit
+        # fixed point (c2_kind = 2) wherever the GEMM takes it: the FFN-up GEMM and the dgrad GEMM that reads it back are
+        # bound by SM store bandwidth / multiplier-tile traffic, and a byte per element carries the same aggregate
+        # gradient error as bf16 (DESIGN.md section 8)
         d, dkind = None, 1
         if act != 0 and tape is not None:
             opA, opB = _operand(xb.ptr, K, False, BF16), _operand(W.shadow.ptr, N, True, BF16)
-            if (GELU_D8 and FUSE_ACT_BWD and act == _lib.ACT["gelu"]
+            if (FUSE_ACT_BWD and act == _lib.ACT["gelu"]
                     and _gemm_tc_supported(M, N, K, opA, opB, y.ptr, N, BF16, bias=b.ptr if b is not None else None, act=act,
                                            c2=y.ptr, c2_kind=2)):
                 d, dkind = Tensor(lead + (N,), U8), 2
@@ -711,66 +704,6 @@ def attention_takes_bias_grad(S, head_dim):
     return bool(FUSED_ATTENTION and head_dim % 8 == 0 and S % 8 == 0 and _lib.call("polus_attention_supported", S, head_dim) == 1)
 
 
-# Dropout keep bits of the attention probabilities, drawn ahead of time.  Per dropout site two persistent device
-# buffers (steps with even / odd optimizer.iterations) + a 2-word "ready" record; created on the first, op-by-op call of a
-# signature (never inside a capture: the record must start zeroed and stay out of the graph's memset nodes).  While a
-# step is being captured, polus_attention_keepbits for step t + 1 is issued on a low-priority background stream right
-# behind the forward kernel of step t: its short CTAs run in the tails of the GEMM waves, and the next replay's forward
-# reads the bits instead of spending 56 % of its instructions on Philox.  The forward checks the record on the device
-# and draws the bits itself when they are not there (first replay, op-by-op execution), so results never depend on it.
-KEEPBITS_AHEAD = _os.environ.get("POLUS_KEEPBITS_AHEAD", "0") != "0"
-_keep_state = {}
-
-
-def invalidate_keep_state():
-    """Forget every published step (the buffers stay: captured graphs hold their addresses).  Called whenever the step
-    counter is rewritten from the host, so bits published for an old trajectory can never be mistaken for the new one's."""
-    for st in _keep_state.values():
-        _lib.call("polus_memset", st[2].ptr, 0, 16, device.stream())
-
-
-reset_keep_state = invalidate_keep_state
-
-
-def capturing():
-    from . import tensor as _t
-    return _t._pool.trace is not None
-
-
-def _keep_buffers(site, Bsz, S, n_heads, p_drop):
-    key = (_rng_state["seed"], site, Bsz, S, n_heads, float(p_drop))
-    st = _keep_state.get(key)
-    if st is None:
-        from . import tensor as _t
-        if _t._pool.trace is not None:
-            return None   # first seen inside a capture (no eager step ran): single graph-owned buffer, drawn in the forward
-        words = int(_lib.call("polus_attention_keepbits_words", Bsz, S, n_heads))
-        st = _keep_state[key] = (device.Buffer(words * 4), device.Buffer(words * 4), device.Buffer(16, zero=True))
-        device.synchronize()
-    return st
-
-
-def rng_stream_fork():
-    """Background stream for work that only has to finish before the optimizer advances the step counter."""
-    if _side.get("rng") is None:
-        s = C.c_void_p()
-        _lib.call("polus_stream_create", C.byref(s), 2)
-        _side["rng"] = s.value
-    ev = _side_event()
-    _lib.call("polus_event_record", ev, device.stream())
-    _lib.call("polus_stream_wait_event", _side["rng"], ev)
-    _side["rng_dirty"] = True
-    return _side["rng"]
-
-
-def rng_stream_join():
-    if _side.get("rng_dirty"):
-        ev = _side_event()
-        _lib.call("polus_event_record", ev, _side["rng"])
-        _lib.call("polus_stream_wait_event", device.stream(), ev)
-        _side["rng_dirty"] = False
-
-
 def _attention_fused(qkv, mask, n_heads, p_drop, qkv_bias=None):
     """One kernel per direction: scores and probabilities stay in TMEM / shared memory (csrc/attention.cu)."""
     Bsz, S, H3 = qkv.shape
@@ -781,26 +714,17 @@ def _attention_fused(qkv, mask, n_heads, p_drop, qkv_bias=None):
     site = _next_site() if p_drop > 0 else 0
     seed = _rng_state["seed"]
     mptr = mask.ptr if mask is not None else None
-    keep = kptr = kalt = ready = None
-    state = _keep_buffers(site, Bsz, S, n_heads, p_drop) if (p_drop > 0 and KEEPBITS_AHEAD) else None
-    if state is not None:
-        kptr, kalt, ready = state[0].ptr, state[1].ptr, state[2].ptr
-    elif p_drop > 0:
-        keep = Tensor((int(_lib.call("polus_attention_keepbits_words", Bsz, S, n_heads)),), I32)
-        kptr = keep.ptr
+    keep = Tensor((int(_lib.call("polus_attention_keepbits_words", Bsz, S, n_heads)),), I32) if p_drop > 0 else None
+    kptr = keep.ptr if keep is not None else None
     _lib.call("polus_attention_fwd", qkv.ptr, mptr, Bsz, S, n_heads, dh, p_drop, seed, site, step_counter(), ctx.ptr,
-              lse.ptr, kptr, kalt, ready, device.stream())
-    if state is not None and capturing():
-        # the NEXT step's bits into the other buffer (this step's backward still reads the current one)
-        _lib.call("polus_attention_keepbits", kptr, kalt, ready, Bsz, S, n_heads, p_drop, seed, site, step_counter(), 1,
-                  rng_stream_fork())
+              lse.ptr, kptr, device.stream())
     tape = _recording(qkv)
     if tape is not None:
-        def backward(g, _alive=(keep, mask, state)):  # the closure uses raw pointers: keep their owners out of the pool
+        def backward(g, _alive=(keep, mask)):  # the closure uses raw pointers: keep their owners out of the pool
             g = cast(g, BF16)
             dqkv = Tensor((Bsz, S, H3), BF16)
             _lib.call("polus_attention_bwd", qkv.ptr, mptr, ctx.ptr, g.ptr, lse.ptr, Bsz, S, n_heads, dh, p_drop, seed, site,
-                      step_counter(), kptr, kalt, dqkv.ptr, qkv_bias.grad.ptr if qkv_bias is not None else None, device.stream())
+                      step_counter(), kptr, dqkv.ptr, qkv_bias.grad.ptr if qkv_bias is not None else None, device.stream())
             return [dqkv]
         _record(tape, [qkv], ctx, backward)
     return ctx

@@ -244,10 +244,6 @@ def reset_arena():
     """Drop every parameter (tests / HPO trials that rebuild models from scratch)."""
     global _arena
     _arena = None
-    import sys
-    ops = sys.modules.get(__name__.rsplit(".", 1)[0] + ".ops")
-    if ops is not None:
-        ops.reset_keep_state()   # per-site dropout buffers of the models that are gone
 
 
 class Param(Tensor):

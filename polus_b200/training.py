@@ -215,7 +215,6 @@ class _CompiledStep:
                 raise RuntimeError("the training step could not be captured into a CUDA graph (an op in the model / loss "
                                    "needs a host<->device sync, e.g. creating a tensor from numpy inside the step); "
                                    "set POLUS_EAGER=1 to run op by op") from e
-            ops.rng_stream_join()   # (a step body that never called tape.gradient still has to join its background work)
             ops.side_join()
             ops.opt_stream_join()
             _lib.call("polus_graph_end", st, C.byref(g))

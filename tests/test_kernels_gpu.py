@@ -400,10 +400,9 @@ def test_gemm_tc_vs_checker_and_host(dev):
 
 @pytest.mark.parametrize("M,N,K,a_mn,b_mn,f32", [(32768, 768, 192, 0, 0, 0), (32768, 768, 136, 0, 1, 0), (32700, 576, 200, 0, 0, 1),
                                                   (32768, 768, 64, 1, 1, 0), (32768, 576, 128, 1, 0, 0), (32768, 768, 3072, 0, 1, 0)])
-def test_gemm_tc_192_wide_pair_tiles(dev, M, N, K, a_mn, b_mn, f32):
-    """192-column pair tiles (opt-in, POLUS_GEMM_BN192=1; the wave cost model picks them for N = 768 / 576 at 32768 rows:
-    6.9 instead of 5.2 waves -- measured slower than 256-wide tiles, so off by default): both operand majors (an MN-major B share of 96 columns is fetched as two 64-column groups), bias, bf16 and
-    fp32 outputs, ragged M and K, column sums -- against numpy fp64."""
+def test_gemm_tc_pair_tiles_ragged_shapes(dev, M, N, K, a_mn, b_mn, f32):
+    """Pair tiles on N = 768 / 576 outputs at about 32768 rows: both operand majors, bias, bf16 and fp32 outputs, ragged
+    M, K and N (576 is not a multiple of 256), column sums -- against numpy fp64."""
     from polus_b200 import _lib
     from polus_b200.tensor import BF16, F32, Tensor
     rng = np.random.default_rng(M + N + K + a_mn)
@@ -421,12 +420,7 @@ def test_gemm_tc_192_wide_pair_tiles(dev, M, N, K, a_mn, b_mn, f32):
     g.accumulate, g.split_k = 0, 1
     if not f32:
         g.colsum = cs_t.ptr
-    import os
-    os.environ["POLUS_GEMM_BN192"] = "1"
-    try:
-        _lib.call("polus_gemm_tc", C.byref(g), st())
-    finally:
-        del os.environ["POLUS_GEMM_BN192"]
+    _lib.call("polus_gemm_tc", C.byref(g), st())
     host = (A.T if a_mn else A).astype(np.float64) @ (B if b_mn else B.T).astype(np.float64) + bias
     out = c_t.numpy().astype(np.float64)
     scale = np.abs(host).max()
@@ -636,14 +630,10 @@ def test_fused_attention_fwd_bwd(dev, B, nh, S, p, use_mask):
     np.testing.assert_allclose(dq_u, dqkv_r, atol=tol_g, rtol=0)
 
 
-# -------------------------------------------------------------------------------------------------- keep bits ahead of time
-def test_attention_keepbits_ahead_bit_exact_and_equivalent(dev):
-    """polus_attention_keepbits (the dropout decisions of the NEXT step, drawn on a background stream) writes exactly the
-    bits the oracle's Philox4x32-10 gives for (seed, site, step + offset) into the buffer of that step's parity and
-    publishes the step; a forward launch that finds them published produces bit-identical output to one that draws them
-    itself, and leaves identical bits for the backward."""
+def test_attention_fwd_keepbits_bit_exact(dev):
+    """The fused forward writes into `keepbits` exactly the dropout decisions the oracle's Philox4x32-10 gives for
+    (seed, site, step), at an even and an odd step: the backward kernel reads them from there."""
     from oracle import philox
-    from polus_b200 import ops
     from polus_b200.tensor import BF16, F32, I32
     B, S, nh, p, seed, site = 2, 128, 3, 0.1, 991, 4
     H = nh * 64
@@ -651,31 +641,9 @@ def test_attention_keepbits_ahead_bit_exact_and_equivalent(dev):
     assert words == B * nh * S * S // 32
     rng = np.random.default_rng(0)
     qkv = T(dev.bf16_round(rng.standard_normal((B, S, 3 * H)).astype(np.float32)), BF16)
-    for step in (6, 7):   # even and odd: both buffers
-        sp = step_ptr(step - 1)                       # the generator runs during step - 1 with offset 1
-        k0, k1, ready = new((words,), I32), new((words,), I32), new((4,), I32)
-        call("polus_attention_keepbits", k0.ptr, k1.ptr, ready.ptr, B, S, nh, p, seed, site, sp, 1, st())
-        buf = k1 if step & 1 else k0
-        got = buf.numpy().view(np.uint32)
+    for step in (6, 7):
         keep = philox.dropout_keep_mask(B * nh * S * S, p, seed, site, step).reshape(-1, 32)
         want = (keep.astype(np.uint32) << np.arange(32, dtype=np.uint32)).sum(1, dtype=np.uint64).astype(np.uint32)
-        assert np.array_equal(got, want)
-        r = ready.numpy().view(np.uint32)
-        assert r[step & 1] == step + 1 and r[(step & 1) ^ 1] == 0
-        assert not (k0 if step & 1 else k1).numpy().any()         # the other buffer was not touched
-        # forward at `step`: (a) bits published ahead, (b) no record -> draws them itself
-        sp = step_ptr(step)
-        ctx_a, ctx_b = new((B, S, H), BF16), new((B, S, H), BF16)
-        lse = new((B, nh, S), F32)
-        call("polus_attention_fwd", qkv.ptr, None, B, S, nh, 64, p, seed, site, sp, ctx_a.ptr, lse.ptr, k0.ptr, k1.ptr, ready.ptr, st())
-        j0, j1 = new((words,), I32), new((words,), I32)
-        call("polus_attention_fwd", qkv.ptr, None, B, S, nh, 64, p, seed, site, sp, ctx_b.ptr, lse.ptr, j0.ptr, j1.ptr, None, st())
-        assert np.array_equal(ctx_a.numpy(), ctx_b.numpy())
-        assert np.array_equal((j1 if step & 1 else j0).numpy().view(np.uint32), want)
-        # a stale record (bits of another step) must be ignored
-        sp = step_ptr(step + 2)
-        ctx_c, ctx_d = new((B, S, H), BF16), new((B, S, H), BF16)
-        call("polus_attention_fwd", qkv.ptr, None, B, S, nh, 64, p, seed, site, sp, ctx_c.ptr, lse.ptr, k0.ptr, k1.ptr, ready.ptr, st())
-        call("polus_attention_fwd", qkv.ptr, None, B, S, nh, 64, p, seed, site, sp, ctx_d.ptr, lse.ptr, j0.ptr, j1.ptr, None, st())
-        assert np.array_equal(ctx_c.numpy(), ctx_d.numpy())
-        assert not np.array_equal(ctx_c.numpy(), ctx_a.numpy())
+        ctx, lse, kb = new((B, S, H), BF16), new((B, nh, S), F32), new((words,), I32)
+        call("polus_attention_fwd", qkv.ptr, None, B, S, nh, 64, p, seed, site, step_ptr(step), ctx.ptr, lse.ptr, kb.ptr, st())
+        assert np.array_equal(kb.numpy().view(np.uint32), want)

@@ -68,7 +68,7 @@ L = 12
 tot += case("fwd_qkv", M, 3 * H, H, op(a, H, 0), op(b, 3 * H, 1), 3 * H, _lib.BF16, count=L)
 tot += case("fwd_attn_out", M, H, H, op(a, H, 0), op(b, H, 1), H, _lib.BF16, count=L)
 tot += case("fwd_ffn1_gelu+gelu'(8-bit)", M, I, H, op(a, H, 0), op(b, I, 1), I, _lib.BF16, act=1, c2=True, c2_kind=2, count=L)
-case("  (fwd_ffn1 gelu + bf16 gelu': POLUS_GELU_D8=0)", M, I, H, op(a, H, 0), op(b, I, 1), I, _lib.BF16, act=1, c2=True, c2_kind=1, count=L)
+case("  (fwd_ffn1 gelu + bf16 gelu')", M, I, H, op(a, H, 0), op(b, I, 1), I, _lib.BF16, act=1, c2=True, c2_kind=1, count=L)
 if os.environ.get("GEMM_EXTRA") == "1":   # what does the FFN-up epilogue pay for: the math, or the two staged stores?
     case("  x1 ffn1 gelu, one output (16-warp)", M, I, H, op(a, H, 0), op(b, I, 1), I, _lib.BF16, act=1, count=L)
     case("  x2 ffn1 no act, C + pre-activation copy (16-warp, no math)", M, I, H, op(a, H, 0), op(b, I, 1), I, _lib.BF16, act=0, c2=True, c2_kind=0, count=L)
@@ -80,7 +80,7 @@ tot += case("dgrad_qkv", M, H, 3 * H, op(a, 3 * H, 0), op(b, 3 * H, 0), H, _lib.
 tot += case("dgrad_attn_out", M, H, H, op(a, H, 0), op(b, H, 0), H, _lib.BF16, use_bias=False, count=L)
 tot += case("dgrad_ffn1", M, H, I, op(a, I, 0), op(b, I, 0), H, _lib.BF16, use_bias=False, count=L)
 tot += case("dgrad_ffn2*gelu'(8-bit)+colsum", M, I, H, op(a, H, 0), op(b, H, 0), I, _lib.BF16, use_bias=False, emul=True, c2_kind=2, count=L)
-case("  (dgrad_ffn2 * bf16 gelu' + colsum: POLUS_GELU_D8=0)", M, I, H, op(a, H, 0), op(b, H, 0), I, _lib.BF16, use_bias=False, emul=True, count=L)
+case("  (dgrad_ffn2 * bf16 gelu' + colsum)", M, I, H, op(a, H, 0), op(b, H, 0), I, _lib.BF16, use_bias=False, emul=True, count=L)
 case("  (same without colsum)", M, I, H, op(a, H, 0), op(b, H, 0), I, _lib.BF16, use_bias=False, emul=True, colsum=False, count=L)
 case("  (plain dgrad_ffn2, no Emul)", M, I, H, op(a, H, 0), op(b, H, 0), I, _lib.BF16, use_bias=False, count=L)
 tot += case("wgrad_qkv", H, 3 * H, M, op(a, H, 1), op(b, 3 * H, 1), 3 * H, _lib.F32, acc=1, split=0, use_bias=False, count=L)

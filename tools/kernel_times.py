@@ -94,10 +94,10 @@ for p_drop in (0.1, 0.0):
     mask = Tensor.from_numpy(np.ones((B, S), np.int32), I32)
     gbq = Tensor((3 * H,), F32, zero=True)
     us = timeit(lambda k: _lib.call("polus_attention_fwd", qkv[k].ptr, mask.ptr, B, S, NH, 64, p_drop, 7, 5, step, ctx[k].ptr, lse.ptr,
-                                    kb.ptr if p_drop else None, None, None, st))
+                                    kb.ptr if p_drop else None, st))
     report(f"attention_fwd p={p_drop}", us, M * H * 2 * 4)
     us = timeit(lambda k: _lib.call("polus_attention_bwd", qkv[k].ptr, mask.ptr, ctx[k].ptr, dctx[k].ptr, lse.ptr, B, S, NH, 64, p_drop, 7, 5,
-                                    step, kb.ptr if p_drop else None, None, dqkv[k].ptr, gbq.ptr, st))
+                                    step, kb.ptr if p_drop else None, dqkv[k].ptr, gbq.ptr, st))
     report(f"attention_bwd p={p_drop}", us, M * H * 2 * 8)
     del qkv, ctx, dctx, dqkv
 
