@@ -935,8 +935,7 @@ extern "C" int polus_attention_bwd(const polus_bf16_t* qkv, const int32_t* mask,
     }
     POLUS_REQUIRE(p_drop == 0.f || d_step != nullptr, "polus_attention_bwd: dropout needs d_step");
     AttnParams p = make_params(B, S, nh, p_drop, seed, site, d_step, mask, const_cast<float*>(lse), const_cast<uint32_t*>(keepbits), gbias_qkv);
-    static const int pf_env = getenv("POLUS_ATTN_PREFETCH") ? atoi(getenv("POLUS_ATTN_PREFETCH")) : 1;
-    p.pf_stride = pf_env > 0 ? pf_env * polus_num_sms() : 0;   // CTA i warms the L2 for CTA i + (number of SMs): one wave ahead
+    p.pf_stride = polus_num_sms();   // CTA i warms the L2 for CTA i + (number of SMs): one wave ahead
     const int n_half = (S + 255) / 256;
     if (n_half > 1) {
         // two CTAs per head (one per 256-query half) add their dK / dV partial sums into dqkv with bf16 TMA reduce-adds:

@@ -52,10 +52,7 @@ int polus_num_sms();
 // kernel launched through polus_launch_pdl() follows: (1) pdl_trigger() first thing, (2) EVERY thread executes
 // pdl_wait() before its first global-memory access that is not to immutable launch arguments.  pdl_wait() returns
 // only when all prerequisite grids have completed and flushed, so ordering stays transitive along the stream.
-// POLUS_PDL=0 turns the launch attribute off (then both instructions are no-ops).
 // ---------------------------------------------------------------------------------------------
-bool polus_pdl_enabled();
-
 template <typename... KArgs, typename... Args>
 inline cudaError_t polus_launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
                                     Args... args) {
@@ -68,7 +65,7 @@ inline cudaError_t polus_launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 bloc
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = polus_pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 

@@ -39,16 +39,11 @@ __device__ __forceinline__ float ksum(float v, int kp) {
     return v;
 }
 
-// KT > 0: the number of tags is the compile-time constant KT (the recursions unroll, E sits in registers, lane indices
-// and shared-memory offsets are immediates); KT == 0: any K <= 32.  With a run-time K every time step re-derived its
-// shared-memory addresses and loop bounds (~100 dependent instructions per step in the SASS).
-template <int KT>
 __global__ void __launch_bounds__(64)
 crf_nll_kernel(const float* __restrict__ emis, const int32_t* __restrict__ tags, const int32_t* __restrict__ lens,
-               const float* __restrict__ trans, const float* __restrict__ weights, int B, int T, int K_rt,
+               const float* __restrict__ trans, const float* __restrict__ weights, int B, int T, int K,
                float* __restrict__ nll_out, float* __restrict__ loss, float* __restrict__ gemis,
                float* __restrict__ gtrans) {
-    const int K = KT > 0 ? KT : K_rt;
     extern __shared__ float sm[];
     float* sE = sm;
     float* sA = sE + K * K;
@@ -83,7 +78,7 @@ crf_nll_kernel(const float* __restrict__ emis, const int32_t* __restrict__ tags,
     float* g = gemis + (long long)b * T * K;
     const bool act = lane < K;
     int kp = 1;
-    while (kp < K) kp <<= 1;  // (a constant when KT > 0)
+    while (kp < K) kp <<= 1;
 
     if (len == 0) {
         for (int i = tid; i < T * K; i += 64) g[i] = 0.f;
@@ -114,21 +109,11 @@ crf_nll_kernel(const float* __restrict__ emis, const int32_t* __restrict__ tags,
         if (act) sAh[lane] = ah;
         if (lane == 0) sC[0] = c;
         float exn = (act && 1 < len) ? sW[K + lane] : 0.f;  // next step's factor, loaded one step ahead
-        float ecol[KT > 0 ? KT : 1];                        // E[i][lane]
-        if (KT > 0) {
-#pragma unroll
-            for (int i = 0; i < KT; ++i) ecol[i] = act ? sE[i * KT + lane] : 0.f;
-        }
         for (int t = 1; t < len; ++t) {
             const float ex = exn;
             exn = (act && t + 1 < len) ? sW[(t + 1) * K + lane] : 0.f;
             float s = 0.f;
-            if (KT > 0) {
-#pragma unroll
-                for (int i = 0; i < KT; ++i) s = fmaf(__shfl_sync(0xffffffffu, ah, i), ecol[i], s);
-            } else {
-                for (int i = 0; i < K; ++i) s = fmaf(__shfl_sync(0xffffffffu, ah, i), act ? sE[i * K + lane] : 0.f, s);
-            }
+            for (int i = 0; i < K; ++i) s = fmaf(__shfl_sync(0xffffffffu, ah, i), act ? sE[i * K + lane] : 0.f, s);
             u = s * ex;
             c = ksum(u, kp);
             ah = u * __frcp_rn(c);
@@ -155,23 +140,13 @@ crf_nll_kernel(const float* __restrict__ emis, const int32_t* __restrict__ tags,
         // ---------------- backward recursion (sW keeps ex_t; w_t[j] = ex_t[j] * beta-tilde_t[j] is rebuilt where it is used)
         float bt = act ? 1.0f : 0.f;  // beta-tilde_{len-1} (any positive constant: marginals renormalise)
         float exn = act ? sW[(len - 1) * K + lane] : 0.f;
-        float erow[KT > 0 ? KT : 1];  // E[lane][j]
-        if (KT > 0) {
-#pragma unroll
-            for (int j = 0; j < KT; ++j) erow[j] = act ? sE[lane * KT + j] : 0.f;
-        }
         for (int t = len - 1; t >= 0; --t) {
             const float wv = exn * bt;  // w_t[j]
             exn = (act && t > 0) ? sW[(t - 1) * K + lane] : 0.f;
             if (act) sBt[t * K + lane] = bt;
             if (t > 0) {
                 float r = 0.f;  // r_{t-1}[i = lane]
-                if (KT > 0) {
-#pragma unroll
-                    for (int j = 0; j < KT; ++j) r = fmaf(erow[j], __shfl_sync(0xffffffffu, wv, j), r);
-                } else {
-                    for (int j = 0; j < K; ++j) r = fmaf(act ? sE[lane * K + j] : 0.f, __shfl_sync(0xffffffffu, wv, j), r);
-                }
+                for (int j = 0; j < K; ++j) r = fmaf(act ? sE[lane * K + j] : 0.f, __shfl_sync(0xffffffffu, wv, j), r);
                 const float d = ksum(r, kp);
                 if (lane == 0) sD[t - 1] = d;
                 bt = r * __frcp_rn(d);
@@ -525,11 +500,9 @@ extern "C" int polus_crf_nll(const float* emis, const int32_t* tags, const int32
     if (B == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     if (loss) POLUS_CHECK_CUDA(cudaMemsetAsync(loss, 0, sizeof(float), st));
-    // K = 4, the polus.ner tag set (PAD, O, B-, I-: polus/ner/utils.py:9-15): one sequence per lane (POLUS_CRF_LANES=0 -> the
-    // tag-per-lane kernel)
-    const char* lanes_s = getenv("POLUS_CRF_LANES");
-    const bool lanes_ok = K == 4 && !(lanes_s && atoi(lanes_s) == 0) &&
-                          ((reinterpret_cast<uintptr_t>(emis) | reinterpret_cast<uintptr_t>(gemis)) & 15) == 0;
+    // K = 4, the polus.ner tag set (PAD, O, B-, I-: polus/ner/utils.py:9-15): one sequence per lane, when its 16-byte row
+    // loads are aligned and four sequences fit in shared memory (T <= 851); otherwise one tag per lane
+    const bool lanes_ok = K == 4 && ((reinterpret_cast<uintptr_t>(emis) | reinterpret_cast<uintptr_t>(gemis)) & 15) == 0;
     auto lanes_smem = [&](int seq) { return ((size_t)48 + (size_t)3 * seq * (T * 4 + 4) + (size_t)3 * seq * (T + 1)) * sizeof(float); };
     if (lanes_ok && lanes_smem(4) <= 200 * 1024) {
         if (lanes_smem(8) <= 200 * 1024) {
@@ -541,12 +514,9 @@ extern "C" int polus_crf_nll(const float* emis, const int32_t* tags, const int32
             if (sz > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_nll_lanes_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sz));
             crf_nll_lanes_kernel<4><<<cdiv(B, 4), 256, sz, st>>>(emis, tags, lens, trans, weights, B, T, nll, loss, gemis, gtrans);
         }
-    } else if (K == 4) {
-        if (smem > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_nll_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        crf_nll_kernel<4><<<B, 64, smem, st>>>(emis, tags, lens, trans, weights, B, T, K, nll, loss, gemis, gtrans);
     } else {
-        if (smem > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_nll_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        crf_nll_kernel<0><<<B, 64, smem, st>>>(emis, tags, lens, trans, weights, B, T, K, nll, loss, gemis, gtrans);
+        if (smem > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_nll_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        crf_nll_kernel<<<B, 64, smem, st>>>(emis, tags, lens, trans, weights, B, T, K, nll, loss, gemis, gtrans);
     }
     g_launch_count++;
     POLUS_LAUNCH_CHECK();

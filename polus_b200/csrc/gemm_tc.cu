@@ -850,7 +850,7 @@ int launch(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, 
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = polus_pdl_enabled() ? 2 : 1;
+    cfg.numAttrs = 2;
     POLUS_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, ta, tb, tc, tc2, p));
     g_launch_count++;
     POLUS_LAUNCH_CHECK();

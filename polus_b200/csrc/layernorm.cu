@@ -136,7 +136,7 @@ ln_res_fwd_kernel(bf16* __restrict__ x, const bf16* __restrict__ res, const floa
 // dbeta = sum dy and (optionally) dbias = sum dx -- the bias gradient of the Dense layer that produced x -- are
 // reduced per CTA in shared memory and added to the gradient arena with one fp32 atomic per column per CTA.
 // keepbits: the forward kernel's dropout decisions (one byte per chunk); NULL => regenerated with Philox.
-template <int NC, bool FULL>
+template <int NC>
 __global__ void __launch_bounds__(kWarps * 32, NC <= 4 ? 2 : 1)
 ln_res_bwd_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ dy2, const bf16* __restrict__ z, const float* __restrict__ mean_in,
                   const float* __restrict__ rstd_in, const float* __restrict__ gamma, int M, int H, DropCfg dc,
@@ -167,7 +167,7 @@ ln_res_bwd_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ dy2, con
 #pragma unroll
         for (int i = 0; i < NC; ++i) {
             const int c = lane + 32 * i;
-            if (FULL || c < chunks) {
+            if (c < chunks) {
                 dyr[i] = ld_stream8(dy + base + c * 8);
                 zr[i] = ld_stream8(z + base + c * 8);
                 if (dc.thresh16 && keepbits != nullptr) kb[i] = keepbits[(long long)row * chunks + c];
@@ -177,7 +177,7 @@ ln_res_bwd_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ dy2, con
 #pragma unroll
             for (int i = 0; i < NC; ++i) {
                 const int c = lane + 32 * i;
-                if (FULL || c < chunks) {
+                if (c < chunks) {
                     float a[8], b2[8];
                     unpack8(dyr[i], a);
                     unpack8(ld_stream8(dy2 + base + c * 8), b2);
@@ -193,7 +193,7 @@ ln_res_bwd_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ dy2, con
 #pragma unroll
         for (int i = 0; i < NC; ++i) {
             const int c = lane + 32 * i;
-            if (FULL || c < chunks) {
+            if (c < chunks) {
                 float dyv[8], zv[8];
                 unpack8(dyr[i], dyv);
                 unpack8(zr[i], zv);
@@ -215,7 +215,7 @@ ln_res_bwd_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ dy2, con
 #pragma unroll
         for (int i = 0; i < NC; ++i) {
             const int c = lane + 32 * i;
-            if (FULL || c < chunks) {
+            if (c < chunks) {
                 float dyv[8], zv[8], dz[8];
                 unpack8(dyr[i], dyv);
                 unpack8(zr[i], zv);
@@ -247,7 +247,7 @@ ln_res_bwd_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ dy2, con
 #pragma unroll
         for (int i = 0; i < NC; ++i) {
             const int c = lane + 32 * i;
-            if (FULL || c < chunks) {
+            if (c < chunks) {
                 float* r8 = red + warp * H + c * 8;
                 const float* src = which == 0 ? dg[i] : (which == 1 ? db[i] : dxs[i]);
                 reinterpret_cast<float4*>(r8)[0] = make_float4(src[0], src[1], src[2], src[3]);
@@ -680,17 +680,16 @@ extern "C" int polus_ln_res_bwd(const polus_bf16_t* dy, const polus_bf16_t* dy2,
     if (grid > kBwdBlocks) grid = kBwdBlocks;
     const size_t smem = (size_t)(kWarps + 1) * H * sizeof(float);
     const int nc = cdiv(H, 256);
-#define LN_BWD(NC_, FULL_)                                                                                                     \
+#define LN_BWD(NC_)                                                                                                            \
     {                                                                                                                          \
-        if (smem > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(ln_res_bwd_kernel<NC_, FULL_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        POLUS_CHECK_CUDA(polus_launch_pdl(ln_res_bwd_kernel<NC_, FULL_>, dim3(grid), dim3(kWarps * 32), smem, st, (const bf16*)dy, (const bf16*)dy2, (const bf16*)z, mean, rstd, gamma, M, H, dc, \
+        if (smem > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(ln_res_bwd_kernel<NC_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        POLUS_CHECK_CUDA(polus_launch_pdl(ln_res_bwd_kernel<NC_>, dim3(grid), dim3(kWarps * 32), smem, st, (const bf16*)dy, (const bf16*)dy2, (const bf16*)z, mean, rstd, gamma, M, H, dc, \
                                           d_step, (bf16*)dx, (bf16*)dres, ggamma, gbeta, gbias_x, keepbits));                  \
     }
     // rows prefetched through shared memory (H = 768: 101 KB per CTA, two CTAs per SM)
-    static const bool pf_env = !(getenv("POLUS_LN_PREFETCH") && atoi(getenv("POLUS_LN_PREFETCH")) == 0);
     const bool aligned = ((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(dy2) | reinterpret_cast<uintptr_t>(z) |
                            reinterpret_cast<uintptr_t>(keepbits)) & 15) == 0;
-    if (pf_env && aligned && (H == 1024 || H == 768 || H == 512 || H == 256)) {
+    if (aligned && (H == 1024 || H == 768 || H == 512 || H == 256)) {
         const size_t smem_pf = (size_t)(kWarps + 1) * H * sizeof(float) + (size_t)kWarps * 2 * (3 * H * 2 + 128) + kWarps * 2 * sizeof(uint64_t);
 #define LN_BWD_PF(NC_)                                                                                                          \
     {                                                                                                                          \
@@ -705,8 +704,7 @@ extern "C" int polus_ln_res_bwd(const polus_bf16_t* dy, const polus_bf16_t* dy2,
         POLUS_LAUNCH_CHECK();
         return 0;
     }
-    if (H == 768) LN_BWD(3, true) else if (H == 1024) LN_BWD(4, true) else if (H == 256) LN_BWD(1, true) else if (H == 512) LN_BWD(2, true)
-    else if (nc <= 1) LN_BWD(1, false) else if (nc == 2) LN_BWD(2, false) else if (nc == 3) LN_BWD(3, false) else if (nc == 4) LN_BWD(4, false) else LN_BWD(16, false)
+    if (nc <= 1) LN_BWD(1) else if (nc == 2) LN_BWD(2) else if (nc == 3) LN_BWD(3) else if (nc == 4) LN_BWD(4) else LN_BWD(16)
 #undef LN_BWD
     g_launch_count++;
     POLUS_LAUNCH_CHECK();

@@ -33,11 +33,6 @@ int polus_num_sms() {
     return g_num_sms;
 }
 
-bool polus_pdl_enabled() {
-    static const bool on = !(getenv("POLUS_PDL") && atoi(getenv("POLUS_PDL")) == 0);
-    return on;
-}
-
 extern "C" {
 
 const char* polus_last_error(void) { return g_err; }

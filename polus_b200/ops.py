@@ -226,9 +226,6 @@ def _accumulate(a, b):
 # they run in those tails and next to the memory-bound LayerNorm / activation-gradient kernels.  Only during
 # capture: there activation blocks are never recycled (tensor._Pool.trace), so the side stream cannot observe a
 # buffer being reused by the main chain.
-import os as _os
-
-SIDE_WGRAD = _os.environ.get("POLUS_SIDE_WGRAD", "1") != "0"
 _side = {"stream": None, "events": [], "next": 0, "dirty": False}
 
 
@@ -244,7 +241,7 @@ def _side_event():
 
 def side_active():
     from . import tensor as _t
-    return SIDE_WGRAD and _t._pool.trace is not None
+    return _t._pool.trace is not None
 
 
 def side_reset():
@@ -438,14 +435,14 @@ def linear(x, W, b=None, activation=None, out_dtype=None, defer_bias_grad=False)
         y = Tensor(lead + (N,), BF16)
         # with an activation the GEMM epilogue also stores act'(z) (not z): backward is then one multiply, which the
         # dgrad GEMM of the layer that consumes y applies in its own epilogue together with the bias-gradient column
-        # sums (FUSE_ACT_BWD) -- no pass over the [M,N] tensor for GeluGrad / BiasAddGrad.  GELU's derivative goes as 8-bit
+        # sums -- no pass over the [M,N] tensor for GeluGrad / BiasAddGrad.  GELU's derivative goes as 8-bit
         # fixed point (c2_kind = 2) wherever the GEMM takes it: the FFN-up GEMM and the dgrad GEMM that reads it back are
         # bound by SM store bandwidth / multiplier-tile traffic, and a byte per element carries the same aggregate
         # gradient error as bf16 (DESIGN.md section 8)
         d, dkind = None, 1
         if act != 0 and tape is not None:
             opA, opB = _operand(xb.ptr, K, False, BF16), _operand(W.shadow.ptr, N, True, BF16)
-            if (FUSE_ACT_BWD and act == _lib.ACT["gelu"]
+            if (act == _lib.ACT["gelu"]
                     and _gemm_tc_supported(M, N, K, opA, opB, y.ptr, N, BF16, bias=b.ptr if b is not None else None, act=act,
                                            c2=y.ptr, c2_kind=2)):
                 d, dkind = Tensor(lead + (N,), U8), 2
@@ -454,7 +451,7 @@ def linear(x, W, b=None, activation=None, out_dtype=None, defer_bias_grad=False)
         _gemm(M, N, K, _operand(xb.ptr, K, False, BF16), _operand(W.shadow.ptr, N, True, BF16),
               y.ptr, N, BF16, bias=b.ptr if b is not None else None, act=act, c2=d.ptr if d is not None else None, c2_kind=dkind)
         if tape is not None:
-            if d is not None and FUSE_ACT_BWD:
+            if d is not None:
                 y.bwd_fuse = (d, b.grad if b is not None else None, dkind)
 
             def backward(g, xb=xb, d=d):
@@ -639,15 +636,30 @@ def layernorm_residual(x, res, gamma, beta, eps=1e-12, p_drop=0.0, x_bias=None):
 def attention(qkv, mask, n_heads, p_drop=0.0, qkv_bias=None):
     """Multi-head self-attention core on the packed projection qkv [B,S,3H] (q|k|v column blocks):
     softmax(QK^T/sqrt(dh) + (1-mask)*-10000) V  ->  ctx [B,S,H]   (HF TFBertSelfAttention; mask constant
-    from polus/models.py:175-195).  Three batched tcgen05 GEMM launches + one softmax launch; the head
-    split/merge transposes of the reference are folded into the TMA tensor maps."""
+    from polus/models.py:175-195).  The fused kernels wherever polus_attention_supported(S, dh) accepts the shape,
+    the GEMM + softmax path otherwise."""
     Bsz, S, H3 = qkv.shape
     H = H3 // 3
     dh = H // n_heads
     assert dh % 8 == 0 and S % 8 == 0, "attention needs head_dim and sequence length multiples of 8"
     qkv = cast(qkv, BF16)
-    if FUSED_ATTENTION and _lib.call("polus_attention_supported", S, dh) == 1:
+    if _lib.call("polus_attention_supported", S, dh) == 1:
         return _attention_fused(qkv, mask, n_heads, p_drop, qkv_bias)
+    return _attention_unfused(qkv, mask, n_heads, p_drop)
+
+
+def attention_takes_bias_grad(S, head_dim):
+    """True when ops.attention(..., qkv_bias=b) will accumulate b's gradient itself (fused kernels): the caller then
+    builds the QKV projection with defer_bias_grad=True."""
+    return bool(head_dim % 8 == 0 and S % 8 == 0 and _lib.call("polus_attention_supported", S, head_dim) == 1)
+
+
+def _attention_unfused(qkv, mask, n_heads, p_drop):
+    """Any S and head_dim (multiples of 8), qkv in bf16.  Three batched tcgen05 GEMM launches + one softmax launch; the
+    head split/merge transposes of the reference are folded into the TMA tensor maps."""
+    Bsz, S, H3 = qkv.shape
+    H = H3 // 3
+    dh = H // n_heads
     nb = Bsz * n_heads
     scale = 1.0 / math.sqrt(dh)
     q_ptr, k_ptr, v_ptr = qkv.ptr, qkv.ptr + H * 2, qkv.ptr + 2 * H * 2
@@ -692,16 +704,6 @@ def attention(qkv, mask, n_heads, p_drop=0.0, qkv_bias=None):
             return [dqkv]
         _record(tape, [qkv], ctx, backward)
     return ctx
-
-
-FUSED_ATTENTION = __import__("os").environ.get("POLUS_FUSED_ATTN", "1") != "0"
-FUSE_ACT_BWD = __import__("os").environ.get("POLUS_FUSE_ACT_BWD", "1") != "0"
-
-
-def attention_takes_bias_grad(S, head_dim):
-    """True when ops.attention(..., qkv_bias=b) will accumulate b's gradient itself (fused kernels): the caller then
-    builds the QKV projection with defer_bias_grad=True."""
-    return bool(FUSED_ATTENTION and head_dim % 8 == 0 and S % 8 == 0 and _lib.call("polus_attention_supported", S, head_dim) == 1)
 
 
 def _attention_fused(qkv, mask, n_heads, p_drop, qkv_bias=None):

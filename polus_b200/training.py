@@ -114,7 +114,6 @@ def _leaf_dtype(x):
     return I32
 
 
-_EARLY_UPDATE = os.environ.get("POLUS_EARLY_UPDATE", "1") != "0"
 _STAGE_SLOTS = 3   # pinned / device staging ring of the input feed
 _copy_stream = [None]
 
@@ -305,7 +304,7 @@ class BaseTrainer:
         # without a gradient post-processing hook nothing reads the full gradient list before the update, so each
         # contiguous span of the arena is updated as soon as backward has finished with it (captured steps only)
         early = None
-        if (self.post_process_grads is None and ops.side_active() and _EARLY_UPDATE
+        if (self.post_process_grads is None and ops.side_active()
                 and hasattr(self.optimizer, "apply_span_early")):
             early = self.optimizer.apply_span_early
         grads = tape.gradient(loss_value, self.trainable_weights, on_bucket_ready=early) if early is not None \

@@ -1,7 +1,7 @@
 #!/bin/bash
 # Marginal cost of each kernel family INSIDE the replayed training-step graph: run bench.py with one family of
-# entry points turned into no-ops (POLUS_ABLATE, polus_b200/_lib.py) and compare ms/step.  Also A/B of the launch
-# features (programmatic dependent launch, background wgrad stream).   usage: tools/ablate_step.sh [out_file]
+# entry points turned into no-ops (POLUS_ABLATE, polus_b200/_lib.py) and compare ms/step.
+# usage: tools/ablate_step.sh [out_file]
 out=${1:-gpurun_out/ablate.txt}
 : > "$out"
 run() {  # label, env...
@@ -10,10 +10,7 @@ run() {  # label, env...
     ms=$(echo "$line" | python -c 'import sys,json; d=json.loads(sys.stdin.read()); print("%.3f ms/step  %.0f seq/s  gemm_frac %.3f" % (d["ms_per_step"], d["value"], d["roofline"]["frac"]))' 2>/dev/null || echo "FAILED")
     printf "%-44s %s\n" "$label" "$ms" | tee -a "$out"
 }
-run "full (pdl=1 side=1)" POLUS_PDL=1 POLUS_SIDE_WGRAD=1
-run "pdl=0 side=1" POLUS_PDL=0 POLUS_SIDE_WGRAD=1
-run "pdl=1 side=0" POLUS_PDL=1 POLUS_SIDE_WGRAD=0
-run "pdl=0 side=0 (previous behaviour)" POLUS_PDL=0 POLUS_SIDE_WGRAD=0
+run "full"
 run "- layernorm fwd+bwd" POLUS_ABLATE=polus_ln_res_fwd,polus_ln_res_bwd
 run "- act_bwd_colsum" POLUS_ABLATE=polus_act_bwd_colsum
 run "- attention fwd+bwd" POLUS_ABLATE=polus_attention_fwd,polus_attention_bwd

@@ -93,8 +93,7 @@ def run(name):
     _lib.call("polus_event_elapsed_ms", e0, e1, C.byref(ms))
     per = ms.value / steps
     sps = batch / (per * 1e-3)
-    from polus_b200 import ops
-    fused = bool(ops.FUSED_ATTENTION and _lib.call("polus_attention_supported", S, 64) == 1)
+    fused = _lib.call("polus_attention_supported", S, 64) == 1
     print(json.dumps({"config": name, "workload": label, "batch": batch, "seq_len": S, "ms_per_step": round(per, 3),
                       "sequences_per_s": round(sps, 1), "step_mfu_vs_sustained_bf16": round(sps * gflop / 1e3 / PEAK, 4),
                       "fused_attention": fused, "launches_per_step": int((_lib.call("polus_launch_count") - l0) / steps),

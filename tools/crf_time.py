@@ -1,5 +1,4 @@
-"""Isolated timing of the CRF loss kernel (polus_crf_nll, K=4, S=256):  python tools/crf_time.py [batch]
-POLUS_CRF_LANES=0 selects the tag-per-lane kernel, the default for K=4 is the sequence-per-lane kernel."""
+"""Isolated timing of the CRF loss kernel (polus_crf_nll, K=4, S=256):  python tools/crf_time.py [batch]"""
 import ctypes as C
 import json
 import os
@@ -41,5 +40,4 @@ device.device_sync()
 ms = C.c_float()
 _lib.call("polus_event_elapsed_ms", e0, e1, C.byref(ms))
 us = ms.value * 1e3 / (REPS * NSETS)
-print(json.dumps({"kernel": "crf_nll K=4", "variant": "tag-per-lane" if os.environ.get("POLUS_CRF_LANES") == "0" else "sequence-per-lane",
-                  "batch": B, "steps": S, "us": round(us, 2), "loss": float(loss.numpy())}), flush=True)
+print(json.dumps({"kernel": "crf_nll K=4", "batch": B, "steps": S, "us": round(us, 2), "loss": float(loss.numpy())}), flush=True)

@@ -5,8 +5,7 @@
 
 Several trials in one process, each a fresh model: the bench's warm-up sequence (op-by-op step, capture, broadcast) and
 `steps` replays with the loss read every 10 steps.  At the first non-finite loss the trial reports which variables,
-gradient spans and optimizer slots hold non-finite values.  Variants toggle the in-graph schedule features
-(early per-span updates, wgrad side stream) to bisect a race."""
+gradient spans and optimizer slots hold non-finite values."""
 import json
 import os
 import sys
@@ -41,10 +40,7 @@ def nonfinite_report(trainer):
     return bad, slots
 
 
-def trial(name, batch, steps, early=True, side=True, check_every=10, workload="ner_base"):
-    from polus_b200 import device, ops, training
-    training._EARLY_UPDATE = early
-    ops.SIDE_WGRAD = side
+def trial(name, batch, steps, check_every=10, workload="ner_base"):
     rank = int(os.environ.get("RANK", "0"))
     trainer, batches, _, _, _ = bench.build_workload(workload, batch)
     t0 = time.time()
@@ -95,11 +91,11 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     device.init(int(os.environ.get("LOCAL_RANK", str(rank))))
     polus_b200.PolusContext()
-    variants = os.environ.get("NANHUNT_VARIANTS", "base,base,base,noearly,noearly,noside,noside").split(",")
+    variants = os.environ.get("NANHUNT_VARIANTS", ",".join(["base"] * 7)).split(",")
     for k, v in enumerate(variants):
-        v, _, wl = v.partition(":")            # "base:cfg4" = default schedule on bench.py's cfg4 workload
+        v, _, wl = v.partition(":")            # "base:cfg4" = bench.py's cfg4 workload
         wl, _, wb = (wl or "ner_base").partition("@")   # "base:cfg5@32" = ... at batch 32
-        trial(f"{v}:{wl}#{k}", int(wb) if wb else batch, steps, early=(v != "noearly" and v != "neither"), side=(v != "noside" and v != "neither"),
+        trial(f"{v}:{wl}#{k}", int(wb) if wb else batch, steps,
               check_every=int(os.environ.get("NANHUNT_CHECK_EVERY", "10")), workload=wl)
     sys.stdout.flush()
     os._exit(0)
