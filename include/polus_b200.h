@@ -223,11 +223,12 @@ int polus_dropout(const polus_bf16_t* d_x, polus_bf16_t* d_y, int64_t n, float p
 /* tfa.text.crf_log_likelihood as used by polus/layers.py:86-126.  Per-sequence nll[b] =
  * log_norm - sequence_score; loss = mean_b(w[b]*nll[b]); gradients of that mean wrt emissions
  * [B,T,K] and transitions [K,K] (accumulated).  d_lens may be NULL (= T for all rows,
- * layers.py:74-76); d_weights may be NULL (= 1).  K <= 32. */
+ * layers.py:74-76); d_weights may be NULL (= 1).  1 <= K <= 128; T up to the shared-memory limit of the
+ * kernel that serves (K, T), at least 512 for every K. */
 int polus_crf_nll(const float* d_emis, const int32_t* d_tags, const int32_t* d_lens,
                   const float* d_trans, const float* d_weights, int B, int T, int K,
                   float* d_nll, float* d_loss, float* d_gemis, float* d_gtrans, void* stream);
-/* tfa.text.crf_decode (polus/layers.py:78-80): Viterbi, ties -> lowest index. */
+/* tfa.text.crf_decode (polus/layers.py:78-80): Viterbi, ties -> lowest index.  Same K and T limits. */
 int polus_crf_decode(const float* d_emis, const int32_t* d_lens, const float* d_trans, int B, int T,
                      int K, int32_t* d_tags, float* d_score, void* stream);
 /* CRF.get_transitions (polus/layers.py:56-63): T*mask + float(int32(1-mask)*-10000) */

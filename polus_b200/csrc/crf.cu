@@ -1,7 +1,9 @@
 // Linear-chain CRF: negative log-likelihood with gradients (forward-backward in one launch) and Viterbi
-// decode.  General K <= 32: one warp per recursion, lane j owns tag j, transitions in shared memory, the T-step
+// decode for K <= 128 tags.  K <= 32: one warp per recursion, lane j owns tag j, transitions in shared memory, the T-step
 // recurrence kept in registers + warp shuffles (crf_nll_kernel, crf_decode_kernel).  K = 4, the polus.ner tag set:
-// one SEQUENCE per lane, the whole K-vector in registers, no cross-lane traffic (crf_nll_lanes_kernel).
+// one SEQUENCE per lane, the whole K-vector in registers, no cross-lane traffic (crf_nll_lanes_kernel).  33 <= K <= 128,
+// and K <= 32 where the [T][K] tables of those kernels do not fit shared memory: one CTA per sequence, thread j owns
+// tag j (crf_nll_wide_kernel, crf_decode_wide_kernel; T up to 19 904 / 1 760 steps at K = 128).
 //
 // Replaces tensorflow_addons.text.crf_log_likelihood / crf_decode, which the reference calls from
 // polus/layers.py:78-80 (decode, also run in training), :91-96 and :109-114 (loss); TF executes them
@@ -457,6 +459,316 @@ __global__ void crf_decode_kernel(const float* __restrict__ emis, const int32_t*
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Wide tag sets (33 <= K <= 128), and K <= 32 at lengths whose [T][K] tables do not fit crf_nll_kernel's or
+// crf_decode_kernel's shared memory (K = 32 at T = 512).  One CTA per sequence, thread j owns tag j (blockDim = K rounded
+// up to 32, padding threads carry zeros).  crf_nll_wide_kernel runs the scaled recursions of crf_nll_kernel one after the
+// other, so that no per-step table lives in shared memory and the kernel needs no workspace:
+//   forward : alpha-hat_t goes to row t of gemis (a [B][T][K] fp32 output anyway); m_t and c_t stay in shared memory.
+//   backward: reads alpha-hat_t back, and overwrites row t with gscale * (gamma_t - onehot(y_t)).
+// Each step broadcasts an unnormalised vector (u_t forward, v_t = ex_t * r_t backward) through shared memory together with
+// the per-warp partial sums of its normaliser, and the reader applies the normaliser: one __syncthreads per step.  The
+// backward works with r_t = beta-tilde_t * d_t, so that g_t = h_t / d_t with h_t = sum_i alpha-hat_t[i] r_t[i], and
+//   gamma_t[i] = alpha-hat_t[i] r_t[i] / h_t,   xi_t[i][j] = alpha-hat_t[i] E[i][j] v_{t+1}[j] / (h_t d_{t+1}).
+// Registers: forward, column j of E (128 floats); backward, row i of sum_t xi_t / E (128 floats), multiplied by E at the end.
+// Shared memory: E [KP][129], KP = blockDim (the backward's row i of E as column i, so that a warp's loads are
+// conflict-free; at the end the transition gradient), m [T], c [T]: (129 KP + 2T) * 4 bytes, 70 KB at K = 128, T = 512.
+constexpr int kWideMaxK = 128;
+constexpr int kWideChunks = kWideMaxK / 32;
+
+__global__ void __launch_bounds__(kWideMaxK)
+crf_nll_wide_kernel(const float* __restrict__ emis, const int32_t* __restrict__ tags, const int32_t* __restrict__ lens,
+                    const float* __restrict__ trans, const float* __restrict__ weights, int B, int T, int K,
+                    float* __restrict__ nll_out, float* __restrict__ loss, float* __restrict__ gemis,
+                    float* __restrict__ gtrans) {
+    extern __shared__ __align__(16) float smw[];
+    constexpr int KS = kWideMaxK + 1;  // a constant stride: the backward's loads of a column of E take immediate offsets
+    const int KP = blockDim.x;
+    float* sE = smw;  // E[i][j] at j * KS + i, zero rows j in [K, KP); after the backward G[i][j] at i * KS + j
+    float* sM = sE + KP * KS;  // [T] m_t = max_j x_t[j]
+    float* sC = sM + T;       // [T] forward normalisers c_t
+    __shared__ __align__(16) float s_vec[3][kWideMaxK];  // broadcast vectors: written at a step, read there and at the next
+    __shared__ float2 s_part[3][kWideChunks];            // their per-warp partial sums
+    const int b = blockIdx.x, j = threadIdx.x, lane = j & 31, warp = j >> 5, nw = blockDim.x >> 5;
+    const bool act = j < K;
+
+    float amax = -INFINITY;
+    for (int i = j; i < K * K; i += blockDim.x) amax = fmaxf(amax, trans[i]);
+    amax = warp_max(amax);
+    if (lane == 0) s_part[2][warp].x = amax;
+    __syncthreads();
+    amax = s_part[2][0].x;
+    for (int w = 1; w < nw; ++w) amax = fmaxf(amax, s_part[2][w].x);
+    for (int idx = j; idx < K * K; idx += blockDim.x) sE[(idx % K) * KS + idx / K] = expf(trans[idx] - amax);
+    for (int idx = K * KS + j; idx < KP * KS; idx += blockDim.x) sE[idx] = 0.f;
+    float e[kWideMaxK];  // E[i][j] for this thread's tag j
+#pragma unroll
+    for (int i = 0; i < kWideMaxK; ++i) e[i] = (act && i < K) ? expf(trans[i * K + j] - amax) : 0.f;
+
+    int len = lens ? lens[b] : T;
+    len = len < 0 ? 0 : (len > T ? T : len);
+    const float gscale = (weights ? weights[b] : 1.0f) / (float)B;
+    const float* x = emis + (long long)b * T * K;
+    const int32_t* y = tags + (long long)b * T;
+    float* g = gemis + (long long)b * T * K;
+    for (int idx = len * K + j; idx < T * K; idx += blockDim.x) g[idx] = 0.f;
+    if (len == 0) {
+        if (j == 0 && nll_out) nll_out[b] = 0.f;
+        return;
+    }
+    for (int t = warp; t < len; t += nw) {  // m_t, one warp per row
+        float m = -INFINITY;
+        for (int q = lane; q < K; q += 32) m = fmaxf(m, x[t * K + q]);
+        m = warp_max(m);
+        if (lane == 0) sM[t] = m;
+    }
+    __syncthreads();
+
+    // ---------------- forward: u_0 = ex_0, u_{t+1}[j] = (sum_i u_t[i] E[i][j]) / c_t * ex_{t+1}[j], c_t = sum_j u_t[j]
+    float u = act ? expf(x[j] - sM[0]) : 0.f;
+    int sl = 0;
+    for (int t = 0;; ++t) {
+        const bool more = t + 1 < len;
+        const float xn = (act && more) ? x[(t + 1) * K + j] : 0.f;  // one step ahead of its use
+        s_vec[sl][j] = u;
+        const float pu = warp_sum(u);
+        if (lane == 0) s_part[sl][warp].x = pu;
+        __syncthreads();
+        float c = s_part[sl][0].x;
+        for (int w = 1; w < nw; ++w) c += s_part[sl][w].x;
+        const float rc = __frcp_rn(c);
+        if (act) g[t * K + j] = u * rc;  // alpha-hat_t
+        if (j == 0) sC[t] = c;
+        if (!more) break;
+        const float* v = s_vec[sl];
+        float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+#pragma unroll
+        for (int ch = 0; ch < kWideChunks; ++ch) {
+            if (ch * 32 < K) {
+#pragma unroll
+                for (int q = ch * 32; q < ch * 32 + 32; q += 4) {
+                    const float4 v4 = *reinterpret_cast<const float4*>(v + q);
+                    s0 = fmaf(v4.x, e[q], s0);
+                    s1 = fmaf(v4.y, e[q + 1], s1);
+                    s2 = fmaf(v4.z, e[q + 2], s2);
+                    s3 = fmaf(v4.w, e[q + 3], s3);
+                }
+            }
+        }
+        u = act ? ((s0 + s1) + (s2 + s3)) * rc * expf(xn - sM[t + 1]) : 0.f;
+        sl = sl == 2 ? 0 : sl + 1;
+    }
+    __syncthreads();
+
+    // ---------------- logZ = sum_t (m_t + log c_t) + (len - 1) max A, and the gold-path score
+    {
+        float lz = 0.f, sc = 0.f;
+        for (int t = j; t < len; t += blockDim.x) {
+            lz += sM[t] + logf(sC[t]);
+            const int yt = min(max(y[t], 0), K - 1);
+            sc += x[t * K + yt];
+            if (t + 1 < len) sc += trans[yt * K + min(max(y[t + 1], 0), K - 1)];
+        }
+        lz = warp_sum(lz);
+        sc = warp_sum(sc);
+        if (lane == 0) s_part[0][warp] = make_float2(lz, sc);
+        s_vec[2][j] = 0.f;  // v_len: the backward's first step has no pair (t, t + 1)
+        __syncthreads();
+        if (j == 0) {
+            float lzs = s_part[0][0].x, scs = s_part[0][0].y;
+            for (int w = 1; w < nw; ++w) {
+                lzs += s_part[0][w].x;
+                scs += s_part[0][w].y;
+            }
+            const float nll = lzs + (float)(len - 1) * amax - scs;
+            if (nll_out) nll_out[b] = nll;
+            if (loss) atomicAdd(loss, nll * gscale);
+        }
+        __syncthreads();
+    }
+
+    // ---------------- backward, thread i = j: r_{len-1} = 1, r_{t-1}[i] = sum_j E[i][j] v_t[j] / d_t, d_t = sum_i r_t[i]
+    const int i = j, il = act ? i : 0;  // padding threads load a valid column and discard the result
+    float gr[kWideMaxK];  // sum_t alpha-hat_t[i] v_{t+1}[j] / (h_t d_{t+1})
+#pragma unroll
+    for (int q = 0; q < kWideMaxK; ++q) gr[q] = 0.f;
+    float r = act ? 1.f : 0.f;
+    float dn = 1.f;  // d_{t+1}
+    float ah = act ? g[(len - 1) * K + i] : 0.f;
+    float xt = act ? x[(len - 1) * K + i] : 0.f;
+    int yt = min(max(y[len - 1], 0), K - 1);
+    int cur = 0, nxt = 2;  // s_vec slots of v_t and v_{t+1}
+    for (int t = len - 1; t >= 0; --t) {
+        float ahp = 0.f, xp = 0.f;
+        int yp = 0;
+        if (t > 0) {  // one step ahead of their use
+            if (act) {
+                ahp = g[(t - 1) * K + i];
+                xp = x[(t - 1) * K + i];
+            }
+            yp = min(max(y[t - 1], 0), K - 1);
+        }
+        s_vec[cur][i] = act ? expf(xt - sM[t]) * r : 0.f;
+        const float pd = warp_sum(r), ph = warp_sum(ah * r);
+        if (lane == 0) s_part[cur][warp] = make_float2(pd, ph);
+        __syncthreads();
+        float d = s_part[cur][0].x, h = s_part[cur][0].y;
+        for (int w = 1; w < nw; ++w) {
+            d += s_part[cur][w].x;
+            h += s_part[cur][w].y;
+        }
+        if (act) g[t * K + i] = gscale * (ah * r * (1.0f / h) - (i == yt ? 1.0f : 0.f));
+        const float coef = (act && t + 1 < len) ? ah / (h * dn) : 0.f;
+        const float* vc = s_vec[cur];
+        const float* vn = s_vec[nxt];
+        float r0 = 0.f, r1 = 0.f, r2 = 0.f, r3 = 0.f;
+#pragma unroll
+        for (int ch = 0; ch < kWideChunks; ++ch) {
+            if (ch * 32 < K) {
+#pragma unroll
+                for (int q = ch * 32; q < ch * 32 + 32; q += 4) {
+                    const float4 c4 = *reinterpret_cast<const float4*>(vc + q);
+                    r0 = fmaf(sE[q * KS + il], c4.x, r0);
+                    r1 = fmaf(sE[(q + 1) * KS + il], c4.y, r1);
+                    r2 = fmaf(sE[(q + 2) * KS + il], c4.z, r2);
+                    r3 = fmaf(sE[(q + 3) * KS + il], c4.w, r3);
+                }
+            }
+        }
+#pragma unroll
+        for (int ch = 0; ch < kWideChunks; ++ch) {
+            if (ch * 32 < K) {
+#pragma unroll
+                for (int q = ch * 32; q < ch * 32 + 32; q += 4) {
+                    const float4 n4 = *reinterpret_cast<const float4*>(vn + q);
+                    gr[q] = fmaf(coef, n4.x, gr[q]);
+                    gr[q + 1] = fmaf(coef, n4.y, gr[q + 1]);
+                    gr[q + 2] = fmaf(coef, n4.z, gr[q + 2]);
+                    gr[q + 3] = fmaf(coef, n4.w, gr[q + 3]);
+                }
+            }
+        }
+        r = act ? ((r0 + r1) + (r2 + r3)) * __frcp_rn(d) : 0.f;
+        dn = d;
+        ah = ahp;
+        xt = xp;
+        yt = yp;
+        nxt = cur;
+        cur = cur == 0 ? 2 : cur - 1;
+    }
+
+    // ---------------- transition gradients: E[i][j] * sum_t ... - counts of gold transitions
+    if (gtrans != nullptr) {
+#pragma unroll
+        for (int q = 0; q < kWideMaxK; ++q)
+            if (act && q < K) gr[q] *= sE[q * KS + i];
+        __syncthreads();
+#pragma unroll
+        for (int q = 0; q < kWideMaxK; ++q)
+            if (act && q < K) sE[i * KS + q] = gr[q];
+        __syncthreads();
+        for (int t = j; t + 1 < len; t += blockDim.x)
+            atomicAdd(&sE[min(max(y[t], 0), K - 1) * KS + min(max(y[t + 1], 0), K - 1)], -1.0f);
+        __syncthreads();
+        for (int idx = j; idx < K * K; idx += blockDim.x) atomicAdd(gtrans + idx, gscale * sE[(idx / K) * KS + idx % K]);
+    }
+}
+
+// Viterbi for the same shapes: thread j owns tag j, keeps column j of A in registers and broadcasts delta_{t-1} through
+// shared memory (one __syncthreads per step).  The max over i runs as four interleaved chains (i mod 4), each keeping its
+// first maximum, merged lowest index first: the same tag and value as one ascending scan with a strict compare, as in
+// crf_decode_kernel.  Back-pointers: u8 [T][K] in shared memory (64 KB at K = 128, T = 512).
+__global__ void __launch_bounds__(kWideMaxK)
+crf_decode_wide_kernel(const float* __restrict__ emis, const int32_t* __restrict__ lens, const float* __restrict__ trans,
+                       int T, int K, int32_t* __restrict__ tags_out, float* __restrict__ score_out) {
+    extern __shared__ uint8_t sbp[];  // [T][K] back-pointers
+    __shared__ __align__(16) float s_delta[2][kWideMaxK];
+    __shared__ float s_bv[kWideChunks];
+    __shared__ int s_bi[kWideChunks];
+    const int b = blockIdx.x, j = threadIdx.x, lane = j & 31, warp = j >> 5, nw = blockDim.x >> 5;
+    const bool act = j < K;
+    int len = lens ? lens[b] : T;
+    len = len < 0 ? 0 : (len > T ? T : len);
+    const float* x = emis + (long long)b * T * K;
+    int32_t* out = tags_out + (long long)b * T;
+    for (int t = len + j; t < T; t += blockDim.x) out[t] = 0;
+    if (len == 0) {
+        if (j == 0 && score_out) score_out[b] = 0.f;
+        return;
+    }
+    float a[kWideMaxK];  // A[i][j]
+#pragma unroll
+    for (int i = 0; i < kWideMaxK; ++i) a[i] = (act && i < K) ? trans[i * K + j] : 0.f;
+    float delta = act ? x[j] : -INFINITY;  // padding tags stay at -inf: never a maximum
+    float xn = (act && 1 < len) ? x[K + j] : 0.f;
+    for (int t = 1; t < len; ++t) {
+        const float xt = xn;
+        if (act && t + 1 < len) xn = x[(t + 1) * K + j];
+        float* dv = s_delta[t & 1];
+        dv[j] = delta;
+        __syncthreads();
+        float bv[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+        int bi[4] = {kWideMaxK, kWideMaxK, kWideMaxK, kWideMaxK};
+#pragma unroll
+        for (int ch = 0; ch < kWideChunks; ++ch) {
+            if (ch * 32 < K) {
+#pragma unroll
+                for (int q = ch * 32; q < ch * 32 + 32; q += 4) {
+                    const float4 d4 = *reinterpret_cast<const float4*>(dv + q);
+                    const float c0 = d4.x + a[q], c1 = d4.y + a[q + 1], c2 = d4.z + a[q + 2], c3 = d4.w + a[q + 3];
+                    if (c0 > bv[0]) { bv[0] = c0; bi[0] = q; }
+                    if (c1 > bv[1]) { bv[1] = c1; bi[1] = q + 1; }
+                    if (c2 > bv[2]) { bv[2] = c2; bi[2] = q + 2; }
+                    if (c3 > bv[3]) { bv[3] = c3; bi[3] = q + 3; }
+                }
+            }
+        }
+#pragma unroll
+        for (int k = 1; k < 4; ++k) {
+            if (bv[k] > bv[0] || (bv[k] == bv[0] && bi[k] < bi[0])) {
+                bv[0] = bv[k];
+                bi[0] = bi[k];
+            }
+        }
+        if (act) {
+            sbp[t * K + j] = (uint8_t)(bi[0] == kWideMaxK ? 0 : bi[0]);  // nothing above -inf: tag 0, as the scan
+            delta = xt + bv[0];
+        }
+    }
+    // final argmax over j, ties -> lowest j
+    float bv = delta;
+    int bi = act ? j : 0x7fffffff;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (ov > bv || (ov == bv && oi < bi)) {
+            bv = ov;
+            bi = oi;
+        }
+    }
+    if (lane == 0) {
+        s_bv[warp] = bv;
+        s_bi[warp] = bi;
+    }
+    __syncthreads();
+    if (j == 0) {
+        for (int w = 1; w < nw; ++w) {
+            if (s_bv[w] > bv || (s_bv[w] == bv && s_bi[w] < bi)) {
+                bv = s_bv[w];
+                bi = s_bi[w];
+            }
+        }
+        if (score_out) score_out[b] = bv;
+        int cur = bi;
+        out[len - 1] = cur;
+        for (int t = len - 1; t >= 1; --t) {
+            cur = sbp[t * K + cur];
+            out[t - 1] = cur;
+        }
+    }
+}
+
 __global__ void crf_mask_kernel(const float* __restrict__ trans, const float* __restrict__ mask, int n, float* __restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = trans[i] * mask[i] + (float)((int)(1.0f - mask[i]) * -10000);
@@ -489,14 +801,22 @@ extern "C" int polus_crf_sample_weights(const float* y_true, const float* mask_p
     return 0;
 }
 
+// Dynamic shared memory the wide kernels may use: the 227 KB a block can opt into, less their static arrays.
+constexpr size_t kWideSmemMax = 220 * 1024;
+
 extern "C" int polus_crf_nll(const float* emis, const int32_t* tags, const int32_t* lens, const float* trans,
                              const float* weights, int B, int T, int K, float* nll, float* loss, float* gemis,
                              float* gtrans, void* stream) {
-    POLUS_REQUIRE(K >= 1 && K <= 32, "polus_crf_nll: K must be in [1,32] (got %d)", K);
+    POLUS_REQUIRE(K >= 1 && K <= kWideMaxK, "polus_crf_nll: K must be in [1,%d] (got %d)", kWideMaxK, K);
     POLUS_REQUIRE(gemis != nullptr, "polus_crf_nll: gemis is required");
     POLUS_REQUIRE(T >= 1, "polus_crf_nll: T must be >= 1");
     const size_t smem = ((size_t)3 * K * K + (size_t)3 * T * K + 2 * (size_t)T) * sizeof(float);
-    POLUS_REQUIRE(smem <= 200 * 1024, "polus_crf_nll: T*K = %d too large for the shared-memory forward-backward tables", T * K);
+    // crf_nll_kernel keeps its [T][K] tables in shared memory; everything else goes to crf_nll_wide_kernel
+    const bool narrow = K <= 32 && smem <= 200 * 1024;
+    const int wide_threads = cdiv(K, 32) * 32;
+    const size_t wide_smem = ((size_t)wide_threads * (kWideMaxK + 1) + 2 * (size_t)T) * sizeof(float);
+    POLUS_REQUIRE(narrow || wide_smem <= kWideSmemMax,
+                  "polus_crf_nll: T = %d too long for the shared-memory tables at K = %d", T, K);
     if (B == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     if (loss) POLUS_CHECK_CUDA(cudaMemsetAsync(loss, 0, sizeof(float), st));
@@ -514,9 +834,13 @@ extern "C" int polus_crf_nll(const float* emis, const int32_t* tags, const int32
             if (sz > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_nll_lanes_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sz));
             crf_nll_lanes_kernel<4><<<cdiv(B, 4), 256, sz, st>>>(emis, tags, lens, trans, weights, B, T, nll, loss, gemis, gtrans);
         }
-    } else {
+    } else if (narrow) {
         if (smem > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_nll_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         crf_nll_kernel<<<B, 64, smem, st>>>(emis, tags, lens, trans, weights, B, T, K, nll, loss, gemis, gtrans);
+    } else {
+        if (wide_smem > 48 * 1024)
+            POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_nll_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wide_smem));
+        crf_nll_wide_kernel<<<B, wide_threads, wide_smem, st>>>(emis, tags, lens, trans, weights, B, T, K, nll, loss, gemis, gtrans);
     }
     g_launch_count++;
     POLUS_LAUNCH_CHECK();
@@ -525,13 +849,23 @@ extern "C" int polus_crf_nll(const float* emis, const int32_t* tags, const int32
 
 extern "C" int polus_crf_decode(const float* emis, const int32_t* lens, const float* trans, int B, int T, int K,
                                 int32_t* tags, float* score, void* stream) {
-    POLUS_REQUIRE(K >= 1 && K <= 32, "polus_crf_decode: K must be in [1,32] (got %d)", K);
+    POLUS_REQUIRE(K >= 1 && K <= kWideMaxK, "polus_crf_decode: K must be in [1,%d] (got %d)", kWideMaxK, K);
     POLUS_REQUIRE(T >= 1, "polus_crf_decode: T must be >= 1");
     const size_t smem = (size_t)K * K * sizeof(float) + (size_t)T * K;
-    POLUS_REQUIRE(smem <= 200 * 1024, "polus_crf_decode: T*K=%d too large for the shared-memory back-pointer table", T * K);
+    // crf_decode_kernel: K <= 32 with A and the back-pointers in shared memory; everything else: crf_decode_wide_kernel
+    const bool narrow = K <= 32 && smem <= 200 * 1024;
+    const size_t wide_smem = (size_t)T * K;
+    POLUS_REQUIRE(narrow || wide_smem <= kWideSmemMax,
+                  "polus_crf_decode: T = %d too long for the shared-memory back-pointer table at K = %d", T, K);
     if (B == 0) return 0;
-    if (smem > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    crf_decode_kernel<<<B, 32, smem, (cudaStream_t)stream>>>(emis, lens, trans, T, K, tags, score);
+    if (narrow) {
+        if (smem > 48 * 1024) POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        crf_decode_kernel<<<B, 32, smem, (cudaStream_t)stream>>>(emis, lens, trans, T, K, tags, score);
+    } else {
+        if (wide_smem > 48 * 1024)
+            POLUS_CHECK_CUDA(cudaFuncSetAttribute(crf_decode_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wide_smem));
+        crf_decode_wide_kernel<<<B, cdiv(K, 32) * 32, wide_smem, (cudaStream_t)stream>>>(emis, lens, trans, T, K, tags, score);
+    }
     g_launch_count++;
     POLUS_LAUNCH_CHECK();
     return 0;

@@ -5,6 +5,9 @@ from . import _lib, device, nn, ops
 from .tensor import F32, I32, Tensor
 
 
+MAX_TAGS = 128  # the largest K that polus_crf_nll / polus_crf_decode accept
+
+
 class CRF(nn.Layer):
     """Linear-chain CRF output layer.
 
@@ -27,6 +30,9 @@ class CRF(nn.Layer):
         self._mask_t = None
 
     def build(self, input_shape):
+        if self.output_dim > MAX_TAGS:
+            raise ValueError(f"CRF supports at most {MAX_TAGS} tags in this port (got output_dim={self.output_dim}); "
+                             "the reference layer (tensorflow_addons) has no such limit")
         if input_shape is not None:
             assert len(input_shape) == 3
             if input_shape[-1] != self.output_dim:
