@@ -160,6 +160,24 @@ int polus_embed_ln_bwd(const polus_bf16_t* d_dy, const float* d_z, const float* 
                        float* d_gpos, float* d_gtype, float* d_ggamma, float* d_gbeta, float* d_ws,
                        void* stream);
 size_t polus_embed_ws_floats(int B, int S, int H); /* size of d_ws above */
+/* The same with per-token position ids (RoBERTa family, or explicit ids): the position row of token (b, s) is
+ * d_pos_ids[b*S + s], clamped to the n_pos rows of d_pos.  Backward adds position gradients keyed by that id; the
+ * padding_idx row receives the gradients of pad tokens (TF semantics).  Available from polus_version() 102. */
+int polus_embed_ln_fwd_pos(const int32_t* d_ids, const int32_t* d_tt, const float* d_word,
+                           const float* d_pos, const float* d_type, const float* d_gamma,
+                           const float* d_beta, int B, int S, int H, int vocab, int n_types, float eps,
+                           float p_drop, uint64_t seed, uint32_t site, const uint32_t* d_step,
+                           polus_bf16_t* d_y, float* d_z, float* d_mean, float* d_rstd,
+                           const int32_t* d_pos_ids, int n_pos, void* stream);
+int polus_embed_ln_bwd_pos(const polus_bf16_t* d_dy, const float* d_z, const float* d_mean,
+                           const float* d_rstd, const float* d_gamma, const int32_t* d_ids,
+                           const int32_t* d_tt, int B, int S, int H, int vocab, int n_types, float p_drop,
+                           uint64_t seed, uint32_t site, const uint32_t* d_step, float* d_gword,
+                           float* d_gpos, float* d_gtype, float* d_ggamma, float* d_gbeta, float* d_ws,
+                           const int32_t* d_pos_ids, int n_pos, void* stream);
+/* HF create_position_ids_from_input_ids on the device: d_pos[b,s] = padding_idx + #(d_ids[b,0..s] != padding_idx)
+ * where d_ids[b,s] != padding_idx, else padding_idx.  [B,S] int32 in and out; no host round trip. */
+int polus_position_ids(const int32_t* d_ids, int B, int S, int padding_idx, int32_t* d_pos, void* stream);
 
 /* HF TFBertSelfOutput / TFBertOutput: y = LN(dropout(x) + res), eps 1e-12.  x is overwritten with
  * z = dropout(x)+res (kept for backward).  res may be NULL. */

@@ -91,6 +91,9 @@ _SIGS = {
     "polus_embed_ln_fwd": [p, p, p, p, p, p, p, i32, i32, i32, i32, i32, f32, f32, u64, u32, p, p, p, p, p, p],
     "polus_embed_ln_bwd": [p, p, p, p, p, p, p, i32, i32, i32, i32, i32, f32, u64, u32, p, p, p, p, p, p, p, p],
     "polus_embed_ws_floats": [i32, i32, i32],
+    "polus_embed_ln_fwd_pos": [p, p, p, p, p, p, p, i32, i32, i32, i32, i32, f32, f32, u64, u32, p, p, p, p, p, p, i32, p],
+    "polus_embed_ln_bwd_pos": [p, p, p, p, p, p, p, i32, i32, i32, i32, i32, f32, u64, u32, p, p, p, p, p, p, p, p, i32, p],
+    "polus_position_ids": [p, i32, i32, i32, p, p],
     "polus_add_bf16": [p, p, p, i64, p],
     "polus_ln_res_fwd": [p, p, p, p, i32, i32, f32, f32, u64, u32, p, p, p, p, p, p],
     "polus_ln_res_bwd": [p, p, p, p, p, p, i32, i32, f32, u64, u32, p, p, p, p, p, p, p, p],

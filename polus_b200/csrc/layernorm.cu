@@ -428,13 +428,35 @@ ln_res_bwd_pf_kernel(const bf16* __restrict__ dy, const bf16* __restrict__ dy2, 
 }
 
 // ------------------------------------------------------------------------------ embeddings
-template <int MAXC>
+// RoBERTa position ids (HF create_position_ids_from_input_ids): padding_idx + (number of non-pad tokens up to and
+// including s) for a real token, padding_idx for a pad token.  One warp per row; the prefix count runs over 32-token
+// slices with a ballot, so any S works and nothing leaves the device.
+__global__ void __launch_bounds__(kWarps * 32)
+position_ids_kernel(const int32_t* __restrict__ ids, int B, int S, int padding_idx, int32_t* __restrict__ pos) {
+    const int lane = threadIdx.x & 31;
+    const int row = blockIdx.x * kWarps + (threadIdx.x >> 5);
+    if (row >= B) return;
+    const int32_t* r = ids + (long long)row * S;
+    int32_t* o = pos + (long long)row * S;
+    int count = padding_idx;
+    for (int s0 = 0; s0 < S; s0 += 32) {
+        const int s = s0 + lane;
+        const bool real = s < S && r[s] != padding_idx;
+        const uint32_t m = __ballot_sync(0xffffffffu, real);
+        if (s < S) o[s] = real ? count + __popc(m & ((2u << lane) - 1u)) : padding_idx;
+        count += __popc(m);
+    }
+}
+
+// POS: the position row of token `row` is pos_ids[row] (clamped to the n_pos rows of the table) instead of row % S.
+template <int MAXC, bool POS>
 __global__ void __launch_bounds__(kWarps * 32)
 embed_ln_fwd_kernel(const int32_t* __restrict__ ids, const int32_t* __restrict__ tt, const float* __restrict__ word,
                     const float* __restrict__ pos, const float* __restrict__ type, const float* __restrict__ gamma,
                     const float* __restrict__ beta, int M, int S, int H, int vocab, int n_types, float eps, DropCfg dc,
                     const uint32_t* __restrict__ d_step, bf16* __restrict__ y, float* __restrict__ zout,
-                    float* __restrict__ mean_out, float* __restrict__ rstd_out) {
+                    float* __restrict__ mean_out, float* __restrict__ rstd_out, const int32_t* __restrict__ pos_ids,
+                    int n_pos) {
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int chunks = H >> 3;
@@ -444,7 +466,13 @@ embed_ln_fwd_kernel(const int32_t* __restrict__ ids, const int32_t* __restrict__
         id = id < 0 ? 0 : (id >= vocab ? vocab - 1 : id);
         int t = tt ? tt[row] : 0;
         t = t < 0 ? 0 : (t >= n_types ? n_types - 1 : t);
-        const int s = row % S;
+        int s;
+        if constexpr (POS) {
+            s = pos_ids[row];
+            s = s < 0 ? 0 : (s >= n_pos ? n_pos - 1 : s);
+        } else {
+            s = row % S;
+        }
         const float* wrow = word + (long long)id * H;
         const float* prow = pos + (long long)s * H;
         const float* trow = type + (long long)t * H;
@@ -587,16 +615,45 @@ embed_ln_bwd_kernel(const bf16* __restrict__ dy, const float* __restrict__ z, co
 // stage B: one CTA per position s.  gpos[s] is owned exclusively (no atomics); token-type sums are
 // reduced in registers (2 types) and word rows are scatter-added with fp32 atomics (what TF's
 // IndexedSlices -> unsorted_segment_sum does for the reference).
+// POS: column s of the batch reaches any position row, keyed by pos_ids (TF semantics: pad tokens add to the
+// padding_idx row like any other).  Two runs of equal position id stay open in registers, the most recently used
+// first; a run is flushed with one atomic per column when a third id evicts it and at the end.  At one s a right- or
+// left-padded batch holds the padding row and, right-padded, one real position: every pad token of the column lands
+// in one register sum instead of one atomic each.
+__device__ __forceinline__ void atomic_add4(float* p, float4 v) {
+    atomicAdd(p + 0, v.x); atomicAdd(p + 1, v.y); atomicAdd(p + 2, v.z); atomicAdd(p + 3, v.w);
+}
+
+template <bool POS>
 __global__ void embed_scatter_kernel(const float* __restrict__ dz, const int32_t* __restrict__ ids,
                                      const int32_t* __restrict__ tt, int B, int S, int H, int vocab, int n_types,
-                                     float* __restrict__ gword, float* __restrict__ gpos, float* __restrict__ gtype) {
+                                     float* __restrict__ gword, float* __restrict__ gpos, float* __restrict__ gtype,
+                                     const int32_t* __restrict__ pos_ids, int n_pos) {
     const int s = blockIdx.x;
     for (int col = threadIdx.x * 4; col < H; col += blockDim.x * 4) {
         float4 accp = make_float4(0.f, 0.f, 0.f, 0.f);
         float4 acct0 = accp, acct1 = accp;
+        float4 acc1 = accp;  // POS: accp is the run of key k0 (most recent), acc1 the run of key k1
+        int k0 = -1, k1 = -1;
         for (int b = 0; b < B; ++b) {
             const long long row = (long long)b * S + s;
             const float4 v = *reinterpret_cast<const float4*>(dz + row * H + col);
+            if constexpr (POS) {
+                int p = pos_ids[row];
+                p = p < 0 ? 0 : (p >= n_pos ? n_pos - 1 : p);
+                if (p != k0) {
+                    if (p != k1) {
+                        if (k1 >= 0 && gpos != nullptr) atomic_add4(gpos + (long long)k1 * H + col, acc1);
+                        k1 = p;
+                        acc1 = make_float4(0.f, 0.f, 0.f, 0.f);
+                    }
+                    const float4 ta = accp;
+                    accp = acc1;
+                    acc1 = ta;
+                    k1 = k0;
+                    k0 = p;
+                }
+            }
             accp.x += v.x; accp.y += v.y; accp.z += v.z; accp.w += v.w;
             if (gword != nullptr) {
                 int id = ids[row];
@@ -613,7 +670,12 @@ __global__ void embed_scatter_kernel(const float* __restrict__ dz, const int32_t
                 atomicAdd(g + 0, v.x); atomicAdd(g + 1, v.y); atomicAdd(g + 2, v.z); atomicAdd(g + 3, v.w);
             }
         }
-        if (gpos != nullptr) {
+        if constexpr (POS) {
+            if (gpos != nullptr) {
+                if (k0 >= 0) atomic_add4(gpos + (long long)k0 * H + col, accp);
+                if (k1 >= 0) atomic_add4(gpos + (long long)k1 * H + col, acc1);
+            }
+        } else if (gpos != nullptr) {
             float4* gp = reinterpret_cast<float4*>(gpos + (long long)s * H + col);
             float4 o = *gp;
             o.x += accp.x; o.y += accp.y; o.z += accp.z; o.w += accp.w;
@@ -715,32 +777,37 @@ extern "C" size_t polus_embed_ws_floats(int B, int S, int H) {
     return (size_t)B * S * H + (size_t)kBwdBlocks * 2 * (size_t)H;
 }
 
-extern "C" int polus_embed_ln_fwd(const int32_t* ids, const int32_t* tt, const float* word, const float* pos,
-                                  const float* type, const float* gamma, const float* beta, int B, int S, int H,
-                                  int vocab, int n_types, float eps, float p_drop, uint64_t seed, uint32_t site,
-                                  const uint32_t* d_step, polus_bf16_t* y, float* z, float* mean, float* rstd, void* stream) {
-    POLUS_REQUIRE(H > 0 && H % 8 == 0 && H <= 4096, "polus_embed_ln_fwd: H must be a multiple of 8 and <= 4096 (got %d)", H);
-    POLUS_REQUIRE(p_drop == 0.f || d_step != nullptr, "polus_embed_ln_fwd: dropout needs d_step");
+namespace {
+
+int embed_fwd(const char* fn, const int32_t* ids, const int32_t* tt, const float* word, const float* pos, const float* type,
+              const float* gamma, const float* beta, int B, int S, int H, int vocab, int n_types, float eps, float p_drop,
+              uint64_t seed, uint32_t site, const uint32_t* d_step, polus_bf16_t* y, float* z, float* mean, float* rstd,
+              const int32_t* pos_ids, int n_pos, void* stream) {
+    POLUS_REQUIRE(H > 0 && H % 8 == 0 && H <= 4096, "%s: H must be a multiple of 8 and <= 4096 (got %d)", fn, H);
+    POLUS_REQUIRE(p_drop == 0.f || d_step != nullptr, "%s: dropout needs d_step", fn);
     const int M = B * S;
     if (M == 0) return 0;
     DropCfg dc = make_drop(p_drop, seed, site);
     cudaStream_t st = (cudaStream_t)stream;
     const int grid = grid_for_rows(M);
-    DISPATCH_MAXC(H,
-        (embed_ln_fwd_kernel<4><<<grid, kWarps * 32, 0, st>>>(ids, tt, word, pos, type, gamma, beta, M, S, H, vocab, n_types, eps, dc, d_step, (bf16*)y, z, mean, rstd)),
-        (embed_ln_fwd_kernel<16><<<grid, kWarps * 32, 0, st>>>(ids, tt, word, pos, type, gamma, beta, M, S, H, vocab, n_types, eps, dc, d_step, (bf16*)y, z, mean, rstd)));
+#define EMB_FWD(MAXC_, POS_) (embed_ln_fwd_kernel<MAXC_, POS_><<<grid, kWarps * 32, 0, st>>>(ids, tt, word, pos, type, gamma, beta, M, S, H, vocab, n_types, eps, dc, d_step, (bf16*)y, z, mean, rstd, pos_ids, n_pos))
+    if (pos_ids != nullptr) {
+        DISPATCH_MAXC(H, EMB_FWD(4, true), EMB_FWD(16, true));
+    } else {
+        DISPATCH_MAXC(H, EMB_FWD(4, false), EMB_FWD(16, false));
+    }
+#undef EMB_FWD
     g_launch_count++;
     POLUS_LAUNCH_CHECK();
     return 0;
 }
 
-extern "C" int polus_embed_ln_bwd(const polus_bf16_t* dy, const float* z, const float* mean, const float* rstd,
-                                  const float* gamma, const int32_t* ids, const int32_t* tt, int B, int S, int H,
-                                  int vocab, int n_types, float p_drop, uint64_t seed, uint32_t site, const uint32_t* d_step,
-                                  float* gword, float* gpos, float* gtype, float* ggamma, float* gbeta, float* ws,
-                                  void* stream) {
-    POLUS_REQUIRE(H > 0 && H % 8 == 0 && H <= 4096, "polus_embed_ln_bwd: H must be a multiple of 8 and <= 4096 (got %d)", H);
-    POLUS_REQUIRE(ws != nullptr, "polus_embed_ln_bwd: workspace required (polus_embed_ws_floats)");
+int embed_bwd(const char* fn, const polus_bf16_t* dy, const float* z, const float* mean, const float* rstd, const float* gamma,
+              const int32_t* ids, const int32_t* tt, int B, int S, int H, int vocab, int n_types, float p_drop, uint64_t seed,
+              uint32_t site, const uint32_t* d_step, float* gword, float* gpos, float* gtype, float* ggamma, float* gbeta,
+              float* ws, const int32_t* pos_ids, int n_pos, void* stream) {
+    POLUS_REQUIRE(H > 0 && H % 8 == 0 && H <= 4096, "%s: H must be a multiple of 8 and <= 4096 (got %d)", fn, H);
+    POLUS_REQUIRE(ws != nullptr, "%s: workspace required (polus_embed_ws_floats)", fn);
     const int M = B * S;
     if (M == 0) return 0;
     DropCfg dc = make_drop(p_drop, seed, site);
@@ -760,7 +827,59 @@ extern "C" int polus_embed_ln_bwd(const polus_bf16_t* dy, const float* z, const 
     }
     g_launch_count++;
     POLUS_LAUNCH_CHECK();
-    embed_scatter_kernel<<<S, 192, 0, st>>>(dz, ids, tt, B, S, H, vocab, n_types, gword, gpos, gtype);
+    if (pos_ids != nullptr)
+        embed_scatter_kernel<true><<<S, 192, 0, st>>>(dz, ids, tt, B, S, H, vocab, n_types, gword, gpos, gtype, pos_ids, n_pos);
+    else
+        embed_scatter_kernel<false><<<S, 192, 0, st>>>(dz, ids, tt, B, S, H, vocab, n_types, gword, gpos, gtype, nullptr, 0);
+    g_launch_count++;
+    POLUS_LAUNCH_CHECK();
+    return 0;
+}
+
+}  // namespace
+
+extern "C" int polus_embed_ln_fwd(const int32_t* ids, const int32_t* tt, const float* word, const float* pos,
+                                  const float* type, const float* gamma, const float* beta, int B, int S, int H,
+                                  int vocab, int n_types, float eps, float p_drop, uint64_t seed, uint32_t site,
+                                  const uint32_t* d_step, polus_bf16_t* y, float* z, float* mean, float* rstd, void* stream) {
+    return embed_fwd("polus_embed_ln_fwd", ids, tt, word, pos, type, gamma, beta, B, S, H, vocab, n_types, eps, p_drop, seed,
+                     site, d_step, y, z, mean, rstd, nullptr, 0, stream);
+}
+
+extern "C" int polus_embed_ln_fwd_pos(const int32_t* ids, const int32_t* tt, const float* word, const float* pos,
+                                      const float* type, const float* gamma, const float* beta, int B, int S, int H,
+                                      int vocab, int n_types, float eps, float p_drop, uint64_t seed, uint32_t site,
+                                      const uint32_t* d_step, polus_bf16_t* y, float* z, float* mean, float* rstd,
+                                      const int32_t* pos_ids, int n_pos, void* stream) {
+    POLUS_REQUIRE(pos_ids != nullptr && n_pos > 0, "polus_embed_ln_fwd_pos: position ids and a table of n_pos > 0 rows required");
+    return embed_fwd("polus_embed_ln_fwd_pos", ids, tt, word, pos, type, gamma, beta, B, S, H, vocab, n_types, eps, p_drop,
+                     seed, site, d_step, y, z, mean, rstd, pos_ids, n_pos, stream);
+}
+
+extern "C" int polus_embed_ln_bwd(const polus_bf16_t* dy, const float* z, const float* mean, const float* rstd,
+                                  const float* gamma, const int32_t* ids, const int32_t* tt, int B, int S, int H,
+                                  int vocab, int n_types, float p_drop, uint64_t seed, uint32_t site, const uint32_t* d_step,
+                                  float* gword, float* gpos, float* gtype, float* ggamma, float* gbeta, float* ws,
+                                  void* stream) {
+    return embed_bwd("polus_embed_ln_bwd", dy, z, mean, rstd, gamma, ids, tt, B, S, H, vocab, n_types, p_drop, seed, site,
+                     d_step, gword, gpos, gtype, ggamma, gbeta, ws, nullptr, 0, stream);
+}
+
+extern "C" int polus_embed_ln_bwd_pos(const polus_bf16_t* dy, const float* z, const float* mean, const float* rstd,
+                                      const float* gamma, const int32_t* ids, const int32_t* tt, int B, int S, int H,
+                                      int vocab, int n_types, float p_drop, uint64_t seed, uint32_t site,
+                                      const uint32_t* d_step, float* gword, float* gpos, float* gtype, float* ggamma,
+                                      float* gbeta, float* ws, const int32_t* pos_ids, int n_pos, void* stream) {
+    POLUS_REQUIRE(pos_ids != nullptr && n_pos > 0, "polus_embed_ln_bwd_pos: position ids and a table of n_pos > 0 rows required");
+    return embed_bwd("polus_embed_ln_bwd_pos", dy, z, mean, rstd, gamma, ids, tt, B, S, H, vocab, n_types, p_drop, seed, site,
+                     d_step, gword, gpos, gtype, ggamma, gbeta, ws, pos_ids, n_pos, stream);
+}
+
+extern "C" int polus_position_ids(const int32_t* ids, int B, int S, int padding_idx, int32_t* pos, void* stream) {
+    POLUS_REQUIRE(B >= 0 && S >= 0, "polus_position_ids: bad shape B=%d S=%d", B, S);
+    if (B == 0 || S == 0) return 0;
+    POLUS_REQUIRE(ids != nullptr && pos != nullptr, "polus_position_ids: ids and pos required");
+    position_ids_kernel<<<cdiv(B, kWarps), kWarps * 32, 0, (cudaStream_t)stream>>>(ids, B, S, padding_idx, pos);
     g_launch_count++;
     POLUS_LAUNCH_CHECK();
     return 0;

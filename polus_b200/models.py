@@ -163,7 +163,8 @@ def bert_model_from_checkpoint(bert_model_checkpoint):
       * a BertModel (returned as is), a BertConfig or a dict of BertConfig fields (random init), or
       * a directory holding `config.json` and, optionally, weights: `weights.npz` (arrays weight0..N in get_weights()
         order, what SavableModel.save writes) or a HuggingFace snapshot's `model.safetensors` (imported with
-        polus_b200.pretrained.load_hf_bert_weights; task heads such as `cls.*` are ignored)."""
+        polus_b200.pretrained.load_hf_bert_weights; task heads such as `cls.*` are ignored).  `model_type` and
+        `pad_token_id` of config.json are kept, so a RoBERTa, XLM-RoBERTa or CamemBERT snapshot gets its position ids."""
     if isinstance(bert_model_checkpoint, BertModel):
         return bert_model_checkpoint
     if isinstance(bert_model_checkpoint, BertConfig):

@@ -70,14 +70,14 @@ class BertNERModel(NERBertModel):
     def sublayers(self):
         return [self.bert, self.dropout, self.hidden, self.out, self.crf]
 
-    def emissions(self, input_ids=None, attention_mask=None, token_type_ids=None, training=False):
+    def emissions(self, input_ids=None, attention_mask=None, token_type_ids=None, training=False, position_ids=None):
         h = self.bert(input_ids=input_ids, attention_mask=attention_mask, token_type_ids=token_type_ids,
-                      training=training)["last_hidden_state"]
+                      training=training, position_ids=position_ids)["last_hidden_state"]
         h = self.dropout(h, training=training)
         return self.out(self.hidden(h, training=training), training=training)
 
-    def call(self, input_ids=None, attention_mask=None, token_type_ids=None, training=False, **unused):
-        e = self.emissions(input_ids, attention_mask, token_type_ids, training=training)
+    def call(self, input_ids=None, attention_mask=None, token_type_ids=None, training=False, position_ids=None, **unused):
+        e = self.emissions(input_ids, attention_mask, token_type_ids, training=training, position_ids=position_ids)
         return self.crf(e, training=training)
 
     def inference(self, x):
@@ -88,7 +88,8 @@ class BertNERModel(NERBertModel):
 @from_config
 def bert_ner_crf(output_classes=4, hidden_space=128, droupout_p=0.1, activation="swish", **kwargs):
     cfg_keys = ("vocab_size", "hidden_size", "num_hidden_layers", "num_attention_heads", "intermediate_size",
-                "max_position_embeddings", "type_vocab_size", "hidden_dropout_prob", "attention_probs_dropout_prob")
+                "max_position_embeddings", "type_vocab_size", "hidden_dropout_prob", "attention_probs_dropout_prob",
+                "layer_norm_eps", "model_type", "pad_token_id")
     cfg = BertConfig(**{k: kwargs[k] for k in cfg_keys if k in kwargs})
     return BertNERModel(cfg, output_classes=output_classes, hidden_space=hidden_space, droupout_p=droupout_p,
                         activation=activation)

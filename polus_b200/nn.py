@@ -238,7 +238,10 @@ class Sequential(Model):
 class BertConfig:
     def __init__(self, vocab_size=30522, hidden_size=768, num_hidden_layers=12, num_attention_heads=12,
                  intermediate_size=3072, max_position_embeddings=512, type_vocab_size=2, hidden_dropout_prob=0.1,
-                 attention_probs_dropout_prob=0.1, layer_norm_eps=1e-12, initializer_range=0.02, **kwargs):
+                 attention_probs_dropout_prob=0.1, layer_norm_eps=1e-12, initializer_range=0.02, model_type="bert",
+                 pad_token_id=0, **kwargs):
+        self.model_type = model_type
+        self.pad_token_id = pad_token_id
         self.vocab_size = vocab_size
         self.hidden_size = hidden_size
         self.num_hidden_layers = num_hidden_layers
@@ -251,6 +254,14 @@ class BertConfig:
         self.layer_norm_eps = layer_norm_eps
         self.initializer_range = initializer_range
         self._name_or_path = kwargs.get("name_or_path", "random-init")
+
+    @property
+    def roberta_positions(self):
+        """RoBERTa-family checkpoints number positions from pad_token_id + 1 and send pad tokens to pad_token_id."""
+        return self.model_type in ROBERTA_MODEL_TYPES
+
+
+ROBERTA_MODEL_TYPES = ("roberta", "xlm-roberta", "camembert")
 
 
 class BertEmbeddings(Layer):
@@ -265,12 +276,25 @@ class BertEmbeddings(Layer):
         self.ln_beta = self.add_weight("LayerNorm/beta", np.zeros(c.hidden_size, np.float32), decay=False)
         self.built = True
 
-    def call(self, input_ids, token_type_ids=None, training=False):
+    def call(self, input_ids, token_type_ids=None, training=False, position_ids=None):
+        """position_ids: int32 [B,S] (HF semantics).  Without them a BERT config uses position s for token s and a
+        RoBERTa-family config derives them from input_ids on the device (pad tokens -> pad_token_id)."""
+        c = self.config
         ids = as_tensor(input_ids, I32)
         tt = as_tensor(token_type_ids, I32) if token_type_ids is not None else None
-        p = self.config.hidden_dropout_prob if training else 0.0
+        if position_ids is not None:
+            pos_ids = as_tensor(position_ids, I32)
+        elif c.roberta_positions:
+            S = ids.shape[1]
+            if S + c.pad_token_id + 1 > c.max_position_embeddings:
+                raise ValueError(f"sequence length {S} needs position ids up to {S + c.pad_token_id} (pad_token_id "
+                                 f"{c.pad_token_id} + 1 + S - 1), beyond the {c.max_position_embeddings} learned positions")
+            pos_ids = ops.position_ids_from_input_ids(ids, c.pad_token_id)
+        else:
+            pos_ids = None
+        p = c.hidden_dropout_prob if training else 0.0
         return ops.embed_layernorm(ids, tt, self.word, self.position, self.token_type, self.ln_gamma, self.ln_beta,
-                                   self.config.layer_norm_eps, p)
+                                   c.layer_norm_eps, p, position_ids=pos_ids)
 
 
 class BertLayer(Layer):
@@ -400,10 +424,10 @@ class BertModel(Model):
     def sublayers(self):
         return [self.bert]
 
-    def call(self, input_ids=None, attention_mask=None, token_type_ids=None, training=False, **unused):
+    def call(self, input_ids=None, attention_mask=None, token_type_ids=None, training=False, position_ids=None, **unused):
         ids = as_tensor(input_ids, I32)
         mask = as_tensor(attention_mask, I32) if attention_mask is not None else None
-        h = self.bert.embeddings(ids, token_type_ids, training=training)
+        h = self.bert.embeddings(ids, token_type_ids, training=training, position_ids=position_ids)
         for layer in self.bert.encoder.layer:
             h = layer(h, attention_mask=mask, training=training)[0]
         out = BertOutput(last_hidden_state=h)

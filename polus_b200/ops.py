@@ -560,30 +560,47 @@ def matmul(a, b, transpose_b=False):
 # ------------------------------------------------------------------------------------------------
 # encoder ops
 # ------------------------------------------------------------------------------------------------
-def embed_layernorm(ids, token_type_ids, word, pos, type_, gamma, beta, eps=1e-12, p_drop=0.0):
-    """HF TFBertEmbeddings (polus/data.py:526-545): LN(word[ids]+pos+type[tt]) -> dropout.  -> bf16 [B,S,H]."""
+def position_ids_from_input_ids(ids, padding_idx):
+    """HF RoBERTa position ids, computed on the device: padding_idx + (count of non-pad tokens up to s) for a real
+    token, padding_idx for a pad token.  int32 [B,S]."""
+    Bsz, S = ids.shape
+    out = Tensor((Bsz, S), I32)
+    _lib.call("polus_position_ids", ids.ptr, Bsz, S, int(padding_idx), out.ptr, device.stream())
+    return out
+
+
+def embed_layernorm(ids, token_type_ids, word, pos, type_, gamma, beta, eps=1e-12, p_drop=0.0, position_ids=None):
+    """HF TFBertEmbeddings (polus/data.py:526-545): LN(word[ids]+pos+type[tt]) -> dropout.  -> bf16 [B,S,H].
+    position_ids: int32 [B,S] rows of `pos` per token (clamped to the table); None = position s for token s."""
     Bsz, S = ids.shape
     V, H = word.shape
     n_types = type_.shape[0]
-    assert S <= pos.shape[0], f"sequence length {S} exceeds the {pos.shape[0]} learned positions"
+    if position_ids is None:
+        assert S <= pos.shape[0], f"sequence length {S} exceeds the {pos.shape[0]} learned positions"
+        fwd, bwd, pos_args = "polus_embed_ln_fwd", "polus_embed_ln_bwd", ()
+    else:
+        assert tuple(position_ids.shape) == (Bsz, S) and position_ids.dtype == I32, "position_ids must be int32 [B,S]"
+        fwd, bwd, pos_args = "polus_embed_ln_fwd_pos", "polus_embed_ln_bwd_pos", (position_ids.ptr, pos.shape[0])
     M = Bsz * S
     y = Tensor((Bsz, S, H), BF16)
     z = Tensor((M, H), F32)
     mean, rstd = Tensor((M,), F32), Tensor((M,), F32)
     site = _next_site() if p_drop > 0 else 0
     seed = _rng_state["seed"]
-    _lib.call("polus_embed_ln_fwd", ids.ptr, token_type_ids.ptr if token_type_ids is not None else None, word.ptr,
+    _lib.call(fwd, ids.ptr, token_type_ids.ptr if token_type_ids is not None else None, word.ptr,
               pos.ptr, type_.ptr, gamma.ptr, beta.ptr, Bsz, S, H, V, n_types, eps, p_drop, seed, site, step_counter(),
-              y.ptr, z.ptr, mean.ptr, rstd.ptr, device.stream())
+              y.ptr, z.ptr, mean.ptr, rstd.ptr, *pos_args, device.stream())
     tape = _recording(word, pos, type_, gamma, beta)
     if tape is not None:
         def backward(g):
             g = cast(g, BF16)
             ws = Tensor((int(_lib.call("polus_embed_ws_floats", Bsz, S, H)),), F32)
-            _lib.call("polus_embed_ln_bwd", g.ptr, z.ptr, mean.ptr, rstd.ptr, gamma.ptr, ids.ptr,
+            # the closure holds position_ids itself, not only its address: it must outlive the forward call
+            pos_args = () if position_ids is None else (position_ids.ptr, pos.shape[0])
+            _lib.call(bwd, g.ptr, z.ptr, mean.ptr, rstd.ptr, gamma.ptr, ids.ptr,
                       token_type_ids.ptr if token_type_ids is not None else None, Bsz, S, H, V, n_types, p_drop, seed,
                       site, step_counter(), word.grad.ptr, pos.grad.ptr, type_.grad.ptr, gamma.grad.ptr, beta.grad.ptr,
-                      ws.ptr, device.stream())
+                      ws.ptr, *pos_args, device.stream())
             return [None] * 5
         _record(tape, [word, pos, type_, gamma, beta], y, backward)
     return y

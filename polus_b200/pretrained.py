@@ -2,7 +2,8 @@
 
 The reference gets pretrained encoders from `TFAutoModel.from_pretrained(checkpoint)` (polus/data.py:526-530,
 polus/models.py:225-229).  Here the weights come from a HuggingFace *state dict* -- a `.safetensors` file, a `.npz`, or a
-mapping name -> array -- with the torch naming (`bert.` prefix optional):
+mapping name -> array -- with the torch naming (`bert.` prefix optional; RoBERTa, XLM-RoBERTa and CamemBERT checkpoints
+use the same names under a `roberta.` prefix, and their heads such as `lm_head.*` are left unused):
 
     embeddings.word_embeddings.weight            [V, H]          encoder.layer.N.attention.output.dense.weight  [H, H]
     embeddings.position_embeddings.weight        [P, H]          encoder.layer.N.attention.output.LayerNorm.*
@@ -31,10 +32,11 @@ def _load_state(source):
 
 
 def load_hf_bert_weights(model, source, strict=True):
-    """Copy a HuggingFace BERT state dict into `model` (a polus_b200.nn.BertModel or its BertMainLayer).
-    Returns the list of state-dict keys that were not used (heads such as `cls.*`)."""
+    """Copy a HuggingFace BERT or RoBERTa-family state dict into `model` (a polus_b200.nn.BertModel or its
+    BertMainLayer).  Returns the list of state-dict keys that were not used (heads such as `cls.*` or `lm_head.*`)."""
     state = _load_state(source)
-    state = {(k[5:] if k.startswith("bert.") else k): v for k, v in state.items()}
+    strip = lambda k: k.split(".", 1)[1] if k.startswith(("bert.", "roberta.")) else k
+    state = {strip(k): v for k, v in state.items()}
     used = set()
 
     def get(name):
