@@ -140,7 +140,9 @@ int polus_skinny_fwd(const void* d_x, int x_dtype, const float* d_W, const float
 /* dx = dz.W^T (may be NULL), gW += x^T.dz, gb += colsum(dz) (may be NULL) */
 int polus_skinny_bwd(const void* d_x, int x_dtype, const float* d_W, const float* d_dz, int M, int K, int N,
                      void* d_dx, int dx_dtype, float* d_gW, float* d_gb, void* stream);
-/* 1 if polus_gemm_tc accepts this problem (alignment / dtype rules), else 0 */
+/* 1 if polus_gemm_tc accepts this problem (alignment / dtype rules), else 0.  N % 8 != 0 (vocabulary projections) is
+ * accepted for plain and bias-only problems with a K-major B (from polus_version() 103).  The contents of C's columns
+ * N .. ldc are unspecified: readers must not use them. */
 int polus_gemm_tc_supported(const polus_gemm_t* g);
 
 /* ---------------------------------------------------------------- memory-bound encoder ops -- */
@@ -264,6 +266,25 @@ int polus_crf_sample_weights(const float* d_y_true, const float* d_mask_positive
 int polus_xent(int kind, const float* d_logits, const void* d_labels, const float* d_class_w,
                float negative_weight, int rows, int C, float* d_loss, float* d_glogits,
                void* stream);
+
+/* ---------------------------------------------------------------- masked-language-model head  */
+/* HF BertForMaskedLM / RobertaForMaskedLM at TF BERT's masked_lm_positions [B,P] (polus_version() >= 103).
+ * Gather: d_out[b*P + j, :] = d_h[b, pos[b,j], :] over bf16 [B,S,H], H % 8 == 0; positions clamped to [0, S).
+ * Scatter: d_dh[b, pos[b,j], :] += d_g[b*P + j, :]; a position named by several slots of a row receives their fp32 sum
+ * (ascending j), rounded to bf16 once.  Deterministic; d_dh is normally zeroed by the caller.  P <= 12288 for the scatter. */
+int polus_gather_positions(const polus_bf16_t* d_h, const int32_t* d_pos, int B, int S, int H, int P,
+                           polus_bf16_t* d_out, void* stream);
+int polus_scatter_positions_add(const polus_bf16_t* d_g, const int32_t* d_pos, int B, int S, int H, int P,
+                                polus_bf16_t* d_dh, void* stream);
+/* Cross-entropy over a vocabulary: bf16 logits [R,V], row stride ldl (>= V, multiple of 8), int32 labels [R] (clamped to
+ * [0,V)), fp32 weights [R].  loss = sum_r w_r (lse_r - x_r[y_r]) / sum_r w_r, 0 when every weight is 0 (fp32 statistics).
+ * Writes d_nll[r] = lse_r - x_r[y_r] and d_argmax[r] (lowest index on ties; may be NULL) and OVERWRITES the logits with
+ * d loss / d logits (bf16; columns V..ldl untouched).  d_labels == NULL: inference, argmax only, logits untouched.
+ * Any V >= 1, one code path. */
+int polus_vocab_xent(polus_bf16_t* d_logits, int R, int V, int64_t ldl, const int32_t* d_labels, const float* d_weights,
+                     float* d_nll, int32_t* d_argmax, float* d_loss, void* stream);
+/* d_out[c] += sum_r d_x[r*ld + c], c < N (bias gradient of the vocabulary projection); one atomic per column per 64-row slab */
+int polus_colsum_bf16(const polus_bf16_t* d_x, int R, int N, int64_t ld, float* d_out, void* stream);
 
 /* ---------------------------------------------------------------- optimizer ----------------- */
 typedef struct {

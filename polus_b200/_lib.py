@@ -112,6 +112,10 @@ _SIGS = {
     "polus_crf_mask_transitions": [p, p, i32, p, p],
     "polus_crf_sample_weights": [p, p, f32, i32, i32, i32, p, p],
     "polus_xent": [i32, p, p, p, f32, i32, i32, p, p, p],
+    "polus_gather_positions": [p, p, i32, i32, i32, i32, p, p],
+    "polus_scatter_positions_add": [p, p, i32, i32, i32, i32, p, p],
+    "polus_vocab_xent": [p, i32, i32, i64, p, p, p, p, p, p],
+    "polus_colsum_bf16": [p, i32, i32, i64, p, p],
     "polus_adam": [p, p, p, p, p, p, i64, C.POINTER(AdamCfg), p, p, i32, p],
     "polus_cast": [p, i32, p, i32, i64, p],
     "polus_fill_f32": [p, f32, i64, p],

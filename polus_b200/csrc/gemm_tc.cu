@@ -927,7 +927,10 @@ const char* why_unsupported(const polus_gemm_t* g) {
         return "batch strides must be multiples of 8 elements";
     const int cvec = g->c_dtype == POLUS_F32 ? 4 : 8;
     if (g->ldc % cvec || g->cbs0 % cvec || g->cbs1 % cvec) return "C strides must be 16-byte multiples";
-    if (g->N % 8) return "N must be a multiple of 8";
+    // N % 8 != 0 (vocabulary projections): the TMA loads of a K-major B zero-fill rows >= N, the epilogue's bias loads
+    // stop at N, and the C tensor map has N columns; C2, Emul, colsum and activations assume whole 8-column groups
+    if (g->N % 8 && (g->B.mn_major || g->C2 || g->Emul || g->colsum || g->c2_kind != 0 || g->act != POLUS_ACT_NONE))
+        return "N not a multiple of 8: only plain or bias-only problems with a K-major B";
     if (g->C2 && (g->c_dtype != POLUS_BF16 || !aligned16(g->C2))) return "C2 requires bf16 C";
     if (g->bias && !aligned16(g->bias)) return "bias must be 16-byte aligned";
     if (g->accumulate && g->c_dtype != POLUS_F32) return "accumulate requires fp32 C";

@@ -437,3 +437,29 @@ class BertModel(Model):
             B, S, H = h.shape
             out["pooler_output"] = ops.gather_rows(ops.reshape(h, (B * S, H)), 0, S, B)
         return out
+
+
+class BertLMPredictionHead(Layer):
+    """HF `cls.predictions` (BERT) / `lm_head` (RoBERTa family): Dense(H, H, gelu) -> LayerNorm -> logits against the TIED
+    word-embedding table plus an output bias [V].  `word_embeddings` is the encoder's word Param, not a copy: the decoder
+    reads its bf16 shadow and adds its gradient into the same fp32 slice as the embedding lookup.
+    Parameters (Keras order): transform kernel [H,H], transform bias, LN gamma, LN beta, output bias [V]."""
+
+    def __init__(self, config, word_embeddings, name="cls/predictions"):
+        super().__init__(name=name)
+        c = self.config = config
+        H, V = c.hidden_size, c.vocab_size
+        assert tuple(word_embeddings.shape) == (V, H), "the decoder is tied to a [vocab_size, hidden_size] table"
+        self.word = word_embeddings
+        self.kernel = self.add_weight("transform/dense/kernel", truncated_normal((H, H), c.initializer_range))
+        self.dense_bias = self.add_weight("transform/dense/bias", np.zeros(H, np.float32), decay=False)
+        self.ln_gamma = self.add_weight("transform/LayerNorm/gamma", np.ones(H, np.float32), decay=False)
+        self.ln_beta = self.add_weight("transform/LayerNorm/beta", np.zeros(H, np.float32), decay=False)
+        self.bias = self.add_weight("bias", np.zeros(V, np.float32), decay=False)
+        self.built = True
+
+    def call(self, hidden_states, training=False):
+        """hidden_states [R, H] (the gathered masked positions) -> bf16 logits [R, V] (ops.VocabLogits)."""
+        t = ops.linear(as_tensor(hidden_states), self.kernel, self.dense_bias, "gelu")
+        t = ops.layernorm_residual(t, None, self.ln_gamma, self.ln_beta, self.config.layer_norm_eps)
+        return ops.vocab_projection(t, self.word, self.bias)

@@ -320,6 +320,9 @@ def zeros(shape, dtype=F32):
 
 def cast(x, dtype):
     """Differentiable dtype conversion."""
+    if isinstance(x, VocabLogits) and x.ld != x.shape[-1]:
+        raise ValueError(f"{x!r} has rows of stride {x.ld}: generic ops read tensors as contiguous (use "
+                         "vocab_cross_entropy / vocab_argmax, or .numpy(), on vocabulary logits)")
     if x.dtype == dtype:
         return x
     out = Tensor(x.shape, dtype)
@@ -786,6 +789,81 @@ def gather_rows(x, first, step, n_rows):
     return out
 
 
+def gather_positions(h, positions):
+    """out[b*P + j] = h[b, positions[b, j]] for bf16 h [B,S,H] and int32 positions [B,P] (TF BERT's masked_lm_positions;
+    clamped to [0, S)).  Backward scatter-adds into a zeroed [B,S,H] gradient; repeated positions sum."""
+    Bsz, S, H = h.shape
+    pos = positions if isinstance(positions, Tensor) else Tensor.from_numpy(np.asarray(positions), I32)
+    if pos.dtype != I32 or pos.ndim != 2 or pos.shape[0] != Bsz:
+        raise ValueError(f"positions must be int32 [B, P] with B = {Bsz}, got {pos.shape}")
+    P = pos.shape[1]
+    h = cast(h, BF16)
+    out = Tensor((Bsz * P, H), BF16)
+    _lib.call("polus_gather_positions", h.ptr, pos.ptr, Bsz, S, H, P, out.ptr, device.stream())
+    tape = _recording(h)
+    if tape is not None:
+        def backward(g, pos=pos):
+            g = cast(g, BF16)
+            dh = Tensor(h.shape, BF16, zero=True)
+            _lib.call("polus_scatter_positions_add", g.ptr, pos.ptr, Bsz, S, H, P, dh.ptr, device.stream())
+            return [dh]
+        _record(tape, [h], out, backward)
+    return out
+
+
+class VocabLogits(Tensor):
+    """bf16 logits [R, V] stored with row stride `ld` = V rounded up to 8 (the GEMM's 16-byte C rows).  Only
+    vocab_cross_entropy, vocab_argmax and .numpy() read it; cast() and view() (so reshape and every op built on them)
+    refuse it when ld != V, instead of reading the padded rows as contiguous."""
+    __slots__ = ("ld",)
+
+    def __init__(self, R, V):
+        ld = (V + 7) // 8 * 8
+        buf = Tensor((R, ld), BF16)
+        Tensor.__init__(self, (R, V), BF16, ptr=buf.ptr, block=buf.block)
+        self.ld = ld
+
+    def view(self, shape):
+        if self.ld != self.shape[1]:
+            raise ValueError(f"vocabulary logits [R, {self.shape[1]}] have rows of stride {self.ld}: no contiguous view")
+        return Tensor.view(self, shape)
+
+    def numpy(self):
+        rows = Tensor((self.shape[0], self.ld), BF16, ptr=self.ptr, block=self.block).numpy()
+        return np.ascontiguousarray(rows[:, :self.shape[1]])
+
+
+def vocab_projection(x, word, bias):
+    """Tied decoder of a masked-LM head: logits[R, V] = x[R, H] . word[V, H]^T + bias, bf16 on the tcgen05 GEMM (any V).
+    `word` is the word-embedding Param (its bf16 shadow is read K-major); its gradient d logits^T . x is reduce-added into
+    word.grad on the side stream during capture, next to the embedding's own scatter-adds."""
+    V, H = word.shape
+    x = cast(x, BF16)
+    R = x.size // H
+    assert x.shape[-1] == H and tuple(bias.shape) == (V,)
+    logits = VocabLogits(R, V)
+    _gemm(R, V, H, _operand(x.ptr, H, False, BF16), _operand(word.shadow.ptr, H, False, BF16), logits.ptr, logits.ld, BF16,
+          bias=bias.ptr)
+    tape = _recording(x, word, bias)
+    if tape is not None:
+        def backward(g):
+            ld = getattr(g, "ld", None)
+            if g.dtype != BF16 or ld is None:
+                raise RuntimeError("vocab_projection's gradient must be the bf16 VocabLogits written by vocab_cross_entropy")
+            _lib.call("polus_colsum_bf16", g.ptr, R, V, ld, bias.grad.ptr, device.stream())
+            # d word[V,H] += g^T . x : A = g (MN-major over V, rows of stride ld), B = x (MN-major over H), reduce over R
+            _gemm(V, H, R, _operand(g.ptr, ld, True, BF16), _operand(x.ptr, H, True, BF16), word.grad.ptr, H, F32,
+                  accumulate=1, split_k=0, stream=side_fork() if side_active() else None)
+            dx = None
+            if x.requires_grad:
+                # dx[R,H] = g[R,V] . word[V,H] : K = V, the TMA loads zero-fill columns >= V of g and rows >= V of word
+                dx = Tensor(x.shape, BF16)
+                _gemm(R, H, V, _operand(g.ptr, ld, False, BF16), _operand(word.shadow.ptr, H, True, BF16), dx.ptr, H, BF16)
+            return [dx, None, None]
+        _record(tape, [x, word, bias], logits, backward)
+    return logits
+
+
 # ------------------------------------------------------------------------------------------------
 # losses
 # ------------------------------------------------------------------------------------------------
@@ -845,6 +923,43 @@ def cross_entropy(kind, logits, labels, class_weights=None, negative_weight=0.0)
     if tape is not None:
         _record(tape, [logits], loss, lambda g: [glog if g.is_one else _scale_by(glog, g)])
     return loss
+
+
+def _vocab_args(logits):
+    if logits.dtype != BF16 or logits.ndim != 2:
+        raise ValueError(f"vocabulary logits must be bf16 [R, V], got {logits!r}")
+    R, V = logits.shape
+    return R, V, getattr(logits, "ld", V)
+
+
+def vocab_cross_entropy(logits, labels, weights):
+    """Masked-LM loss sum_r w_r (lse_r - x_r[y_r]) / sum_r w_r over bf16 logits [R, V] (0 when every weight is 0).
+    Returns (loss, argmax [R] int32).  The kernel writes d loss / d logits over the logits in place (read them before
+    calling this), which is what the backward hands to the decoder GEMMs.  It must be the loss the tape starts from."""
+    R, V, ld = _vocab_args(logits)
+    labels = labels if isinstance(labels, Tensor) else Tensor.from_numpy(np.asarray(labels), I32)
+    weights = weights if isinstance(weights, Tensor) else Tensor.from_numpy(np.asarray(weights), F32)
+    weights = cast(weights, F32)
+    if labels.dtype != I32 or labels.size != R or weights.size != R:
+        raise ValueError(f"labels (int32) and weights need {R} entries, got {labels!r} and {weights!r}")
+    loss, nll, amax = Tensor((), F32), Tensor((R,), F32), Tensor((R,), I32)
+    _lib.call("polus_vocab_xent", logits.ptr, R, V, ld, labels.ptr, weights.ptr, nll.ptr, amax.ptr, loss.ptr, device.stream())
+    tape = _recording(logits)
+    if tape is not None:
+        def backward(g):
+            if not g.is_one:
+                raise RuntimeError("vocab_cross_entropy writes its gradient for d loss = 1: use it as the loss itself")
+            return [logits]
+        _record(tape, [logits], loss, backward)
+    return loss, amax
+
+
+def vocab_argmax(logits):
+    """int32 [R]: the highest logit of each row, lowest index on ties (logits untouched)."""
+    R, V, ld = _vocab_args(logits)
+    out = Tensor((R,), I32)
+    _lib.call("polus_vocab_xent", logits.ptr, R, V, ld, None, None, None, out.ptr, None, device.stream())
+    return out
 
 
 # ------------------------------------------------------------------------------------------------
