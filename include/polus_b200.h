@@ -144,6 +144,11 @@ int polus_skinny_bwd(const void* d_x, int x_dtype, const float* d_W, const float
  * accepted for plain and bias-only problems with a K-major B (from polus_version() 103).  The contents of C's columns
  * N .. ldc are unspecified: readers must not use them. */
 int polus_gemm_tc_supported(const polus_gemm_t* g);
+/* The kernel polus_gemm_tc launches for this problem, without launching it: out4 = {CTAs per tile (1, or 2 for a CTA
+ * pair on 256-row tiles), tile width BN (64, 128 or 256), K splits as launched, 1 if the 16-epilogue-warp kernel runs}.
+ * With the operand majors this names the kernel instantiation.  Fails like polus_gemm_tc on an unsupported problem.
+ * Available from polus_version() 104. */
+int polus_gemm_tc_plan(const polus_gemm_t* g, int* out4);
 
 /* ---------------------------------------------------------------- memory-bound encoder ops -- */
 /* Dropout sites are addressed by (seed, site, *d_step): Philox4x32-10 counters, no stored masks. */

@@ -85,6 +85,7 @@ _SIGS = {
     "polus_gemm_tc": [C.POINTER(Gemm), p],
     "polus_gemm_small": [C.POINTER(Gemm), p],
     "polus_gemm_tc_supported": [C.POINTER(Gemm)],
+    "polus_gemm_tc_plan": [C.POINTER(Gemm), C.POINTER(i32)],
     "polus_skinny_supported": [i32, i32],
     "polus_skinny_fwd": [p, i32, p, p, i32, i32, i32, i32, p, p, p],
     "polus_skinny_bwd": [p, i32, p, p, i32, i32, i32, p, i32, p, p, p],

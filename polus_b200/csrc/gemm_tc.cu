@@ -542,6 +542,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         __syncwarp();  // every lane has its multipliers: the tile may be refilled
                         advance(pf_t, pf_i);
                         if (pf_t < p.num_tiles) emul_issue(pf_t, pf_i, ebuf);
+                    } else if (p.has_c2 && p.c2_grad) {
+                        // activation + derivative on the partial last block (N % 32 != 0; only bf16 derivatives get here)
+#pragma unroll
+                        for (int j = 0; j < 4; ++j) {
+                            float d8[8];
+                            act_fwd_grad8(p.act, v + 8 * j, d8);
+                            sts16(sX, j, d8);
+                        }
                     } else {
                         if (p.has_c2) {
 #pragma unroll
@@ -918,6 +926,23 @@ TilePlan plan_tiles(const polus_gemm_t* g, int sms) {
     return t;
 }
 
+struct SplitK {
+    int kb_total;      // 64-deep k-blocks of the problem
+    int kb_per_split;  // k-blocks per split
+    int split_k;       // splits launched: none of them empty
+};
+
+// The split the kernel runs for a planned split: at most one split per k-block, and the count recomputed from the
+// k-blocks per split so that the last split is never empty.
+SplitK clamp_split(int split, int K) {
+    SplitK s;
+    s.kb_total = cdiv(K, BK);
+    if (split > s.kb_total) split = s.kb_total;
+    s.kb_per_split = cdiv(s.kb_total, split);
+    s.split_k = cdiv(s.kb_total, s.kb_per_split);
+    return s;
+}
+
 const char* why_unsupported(const polus_gemm_t* g) {
     if (g->A.dtype != POLUS_BF16 || g->B.dtype != POLUS_BF16) return "operands must be bf16";
     if (g->M < 1 || g->N < 1 || g->K < 1) return "empty problem";
@@ -955,6 +980,17 @@ const char* why_unsupported(const polus_gemm_t* g) {
 
 extern "C" int polus_gemm_tc_supported(const polus_gemm_t* g) { return why_unsupported(g) == nullptr ? 1 : 0; }
 
+extern "C" int polus_gemm_tc_plan(const polus_gemm_t* g, int* out4) {
+    const char* why = why_unsupported(g);
+    POLUS_REQUIRE(why == nullptr, "polus_gemm_tc_plan: unsupported problem (%s) M=%d N=%d K=%d", why, g->M, g->N, g->K);
+    const TilePlan plan = plan_tiles(g, polus_num_sms());
+    out4[0] = plan.CG;
+    out4[1] = plan.BN;
+    out4[2] = clamp_split(plan.split, g->K).split_k;
+    out4[3] = plan.epi16 ? 1 : 0;
+    return 0;
+}
+
 extern "C" int polus_gemm_tc(const polus_gemm_t* g, void* stream) {
     const char* why = why_unsupported(g);
     POLUS_REQUIRE(why == nullptr, "polus_gemm_tc: unsupported problem (%s) M=%d N=%d K=%d", why, g->M, g->N, g->K);
@@ -964,7 +1000,7 @@ extern "C" int polus_gemm_tc(const polus_gemm_t* g, void* stream) {
     const int CG = plan.CG, BN = plan.BN;
     const long long mt = cdiv(g->M, BM * CG);
     const long long nb = (long long)batch0 * batch1;
-    int split = plan.split;
+    const SplitK split = clamp_split(plan.split, g->K);
 
     TcParams p;
     p.M = g->M;
@@ -973,10 +1009,9 @@ extern "C" int polus_gemm_tc(const polus_gemm_t* g, void* stream) {
     p.batch0 = batch0;
     p.m_tiles = (int)mt;
     p.n_tiles = cdiv(g->N, BN);
-    p.kb_total = cdiv(g->K, BK);
-    if (split > p.kb_total) split = p.kb_total;
-    p.kb_per_split = cdiv(p.kb_total, split);
-    p.split_k = cdiv(p.kb_total, p.kb_per_split);
+    p.kb_total = split.kb_total;
+    p.kb_per_split = split.kb_per_split;
+    p.split_k = split.split_k;
     p.num_tiles = (int)(mt * p.n_tiles * p.split_k * nb);
     // Rasterisation: concurrently running tiles form (about) an 8 x 9 patch of the tile grid instead of a 74 x 1 column
     // strip, so each A row block and each B column block in flight is shared by 8-9 clusters (measured 1.05-1.15x).

@@ -711,6 +711,8 @@ extern "C" int polus_ln_res_fwd(polus_bf16_t* x, const polus_bf16_t* res, const 
     POLUS_REQUIRE(M >= 0 && H > 0 && H % 8 == 0 && H <= 4096, "polus_ln_res_fwd: H must be a multiple of 8 and <= 4096 (got %d)", H);
     POLUS_REQUIRE(p_drop >= 0.f && p_drop < 1.f, "polus_ln_res_fwd: bad dropout %f", p_drop);
     POLUS_REQUIRE(p_drop == 0.f || d_step != nullptr, "polus_ln_res_fwd: dropout needs d_step");
+    POLUS_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(res) | reinterpret_cast<uintptr_t>(y)) & 15) == 0,
+                  "polus_ln_res_fwd: x, res and y must be 16-byte aligned");
     if (M == 0) return 0;
     DropCfg dc = make_drop(p_drop, seed, site);
     cudaStream_t st = (cudaStream_t)stream;
@@ -735,6 +737,10 @@ extern "C" int polus_ln_res_bwd(const polus_bf16_t* dy, const polus_bf16_t* dy2,
     POLUS_REQUIRE(M >= 0 && H > 0 && H % 8 == 0 && H <= 4096, "polus_ln_res_bwd: H must be a multiple of 8 and <= 4096 (got %d)", H);
     POLUS_REQUIRE(dx != nullptr, "polus_ln_res_bwd: dx required");
     POLUS_REQUIRE(!(p_drop > 0.f && dres == dx), "polus_ln_res_bwd: dres may alias dx only without dropout");
+    // both kernels move rows in 16-byte vectors; only keepbits (read bytewise by ln_res_bwd_kernel) may be less aligned
+    POLUS_REQUIRE(((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(dy2) | reinterpret_cast<uintptr_t>(z) |
+                    reinterpret_cast<uintptr_t>(dx) | reinterpret_cast<uintptr_t>(dres)) & 15) == 0,
+                  "polus_ln_res_bwd: dy, dy2, z, dx and dres must be 16-byte aligned");
     if (M == 0) return 0;
     DropCfg dc = make_drop(p_drop, seed, site);
     cudaStream_t st = (cudaStream_t)stream;
@@ -748,10 +754,10 @@ extern "C" int polus_ln_res_bwd(const polus_bf16_t* dy, const polus_bf16_t* dy2,
         POLUS_CHECK_CUDA(polus_launch_pdl(ln_res_bwd_kernel<NC_>, dim3(grid), dim3(kWarps * 32), smem, st, (const bf16*)dy, (const bf16*)dy2, (const bf16*)z, mean, rstd, gamma, M, H, dc, \
                                           d_step, (bf16*)dx, (bf16*)dres, ggamma, gbeta, gbias_x, keepbits));                  \
     }
-    // rows prefetched through shared memory (H = 768: 101 KB per CTA, two CTAs per SM)
-    const bool aligned = ((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(dy2) | reinterpret_cast<uintptr_t>(z) |
-                           reinterpret_cast<uintptr_t>(keepbits)) & 15) == 0;
-    if (aligned && (H == 1024 || H == 768 || H == 512 || H == 256)) {
+    // rows prefetched through shared memory (H = 768: 101 KB per CTA, two CTAs per SM); the keep bytes ride on the same
+    // bulk copies, which need 16-byte alignment
+    const bool kb_aligned = (reinterpret_cast<uintptr_t>(keepbits) & 15) == 0;
+    if (kb_aligned && (H == 1024 || H == 768 || H == 512 || H == 256)) {
         const size_t smem_pf = (size_t)(kWarps + 1) * H * sizeof(float) + (size_t)kWarps * 2 * (3 * H * 2 + 128) + kWarps * 2 * sizeof(uint64_t);
 #define LN_BWD_PF(NC_)                                                                                                          \
     {                                                                                                                          \

@@ -36,7 +36,7 @@ int polus_num_sms() {
 extern "C" {
 
 const char* polus_last_error(void) { return g_err; }
-int polus_version(void) { return 103; }
+int polus_version(void) { return 104; }
 
 int polus_device_count(int* n) {
     POLUS_CHECK_CUDA(cudaGetDeviceCount(n));

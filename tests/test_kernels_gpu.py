@@ -62,7 +62,12 @@ BF16_EPS = 2.0 ** -8
 
 # --------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("M,H,p", [(64, 768, 0.0), (37, 128, 0.0), (50, 1024, 0.1), (8, 2048, 0.0), (0, 768, 0.0),
-                                   (21, 384, 0.1), (33, 640, 0.0), (29, 1000, 0.1)])
+                                   (21, 384, 0.1), (33, 640, 0.0), (29, 1000, 0.1),
+                                   # several rows per warp: the backward's 296 CTAs x 8 warps take a second row past
+                                   # M = 2368 (7109 = three row strides + 5), the forward's 2368 x 4 warps past 9472
+                                   (7109, 256, 0.1), (20000, 256, 0.0), (7109, 512, 0.0), (20000, 512, 0.1),
+                                   (7109, 768, 0.1), (20000, 768, 0.0), (7109, 1024, 0.0), (20000, 1024, 0.1),
+                                   (5000, 4096, 0.1)])
 def test_ln_residual_fwd_bwd(dev, M, H, p):
     from oracle import numpy_ref as R, philox
     from polus_b200.tensor import BF16, F32
@@ -571,62 +576,8 @@ def test_skinny_linear_fwd_bwd(dev, M, K, N, act, xdt):
 def test_fused_attention_fwd_bwd(dev, B, nh, S, p, use_mask):
     """Fused attention (scores/probabilities in TMEM/smem) vs the oracle with the device's own dropout masks, and vs
     the unfused GEMM+softmax path (same Philox counters => same masks)."""
-    from oracle import numpy_ref as R, philox
-    from polus_b200 import ops
-    from polus_b200.tensor import BF16, I32, Tensor
-    rng = np.random.default_rng(S + nh)
-    dh, H = 64, nh * 64
-    qkv = dev.bf16_round(rng.standard_normal((B, S, 3 * H)).astype(np.float32))
-    dctx = dev.bf16_round(rng.standard_normal((B, S, H)).astype(np.float32))
-    lens = rng.integers(max(S // 2, 1), S + 1, B)
-    mask = (np.arange(S)[None] < lens[:, None]).astype(np.int32)
-    ops.set_seed(77)
-    ops.set_step(3)
-
-    from polus_b200.tensor import Param
-    bias = Param(np.zeros(3 * H, np.float32), name="qkv_bias")  # only its .grad is touched
-
-    def run(fused):
-        ops.reset_dropout_sites()
-        x = Tensor.from_numpy(qkv, BF16)
-        x.requires_grad = True
-        m = Tensor.from_numpy(mask, I32) if use_mask else None
-        with ops.GradientTape() as tape:
-            ctx = ops.attention(x, m, nh, p, qkv_bias=bias) if fused else ops._attention_unfused(x, m, nh, p)
-        # seed the backward with dctx: d(sum(ctx*dctx))
-        tape.nodes[-1].output = ctx
-        g = tape.nodes[-1].backward(Tensor.from_numpy(dctx, BF16))[0]
-        return ctx.numpy(), g.numpy()
-    ctx_f, dq_f = run(True)
-    ctx_u, dq_u = run(False)
-    # the fused backward also accumulates the QKV bias gradient = column sums of the dqkv it stored
-    gb_ref = dq_f.astype(np.float64).reshape(-1, 3 * H).sum(0)
-    if S <= 256:
-        np.testing.assert_allclose(bias.grad.numpy(), gb_ref, rtol=1e-4, atol=1e-4 * (np.abs(gb_ref).max() + 1))
-    else:
-        # two CTAs per head: the bias sums add each half's bf16 partial dK / dV, the stored tensor holds the bf16 sum of
-        # the two partials -- they differ by that final rounding (<= 2^-9 |x| per element, worst case over the column)
-        bound = 2.0 ** -9 * np.abs(dq_f.astype(np.float64)).reshape(-1, 3 * H).sum(0) + 1e-4 * (np.abs(gb_ref).max() + 1)
-        assert np.all(np.abs(bias.grad.numpy() - gb_ref) <= bound)
-    # oracle (float64) with the same dropout mask (site 1 of this step)
-    q, k, v = [qkv[..., i * H:(i + 1) * H].reshape(B, S, nh, dh).transpose(0, 2, 1, 3).astype(np.float64) for i in range(3)]
-    sc = q @ k.transpose(0, 1, 3, 2) / 8.0 + (R.attention_mask_additive(mask) if use_mask else 0.0)
-    P = R.softmax(sc)
-    dm = philox.dropout_scale_mask((B, nh, S, S), p, 77, 1, 3).astype(np.float64) if p > 0 else 1.0
-    Pd = P * dm
-    ctx_r = (Pd @ v).transpose(0, 2, 1, 3).reshape(B, S, H)
-    do = dctx.reshape(B, S, nh, dh).transpose(0, 2, 1, 3).astype(np.float64)
-    dPd = do @ v.transpose(0, 1, 3, 2)
-    dv = Pd.transpose(0, 1, 3, 2) @ do
-    dP = dPd * dm
-    dS = P * (dP - (P * dP).sum(-1, keepdims=True)) / 8.0
-    dq, dk = dS @ k, dS.transpose(0, 1, 3, 2) @ q
-    dqkv_r = np.concatenate([t.transpose(0, 2, 1, 3).reshape(B, S, H) for t in (dq, dk, dv)], -1)
-    tol_c, tol_g = 2e-2 * np.abs(ctx_r).max(), 2e-2 * np.abs(dqkv_r).max()
-    np.testing.assert_allclose(ctx_f, ctx_r, atol=tol_c, rtol=0)
-    np.testing.assert_allclose(dq_f, dqkv_r, atol=tol_g, rtol=0)
-    np.testing.assert_allclose(ctx_u, ctx_r, atol=tol_c, rtol=0)
-    np.testing.assert_allclose(dq_u, dqkv_r, atol=tol_g, rtol=0)
+    from tests.attention_ref import check_attention_case
+    check_attention_case(dev, B, nh, S, p, use_mask)
 
 
 def test_attention_fwd_keepbits_bit_exact(dev):
